@@ -6,6 +6,7 @@ batch of windows per GPU (weak scaling: every rank owns its own batch; the eval 
 Default workload = BASELINE.json configs[1], the shape the metric is quoted on: (B,N,W,H)=(32,358,12,3).
 
     python bench.py [--gpus N --steps K --warmup W] [--config cfg1..cfg5]     # this repo's CUDA path
+    python bench.py ... --dump-outputs DIR       # also write the last timed step's forecast / attention as DIR/*.npy
     python bench.py --impl reference [...]                                    # the reference's own CPU path
 
 Prints ONE JSON line.  Keys (see the task contract):
@@ -17,8 +18,11 @@ Prints ONE JSON line.  Keys (see the task contract):
                         between this forward and the reference's CPU forward on the SAME inputs/weights
   roofline              the dominant kernel (GRU recurrence), timed live with CUDA events via the
                         library's stemgnn_profile_gru hook; flops = SURVEY.md §8(d) GRU terms
-  cpu_baseline          the unmodified reference (baseline/_ref or /root/reference under oracle/ref_shim.py;
-                        kind "reference") — or the torch port when no copy is present (kind "port") — on the host cores
+  cpu_baseline          the unmodified reference (the checkout named by STEMGNN_REFERENCE_ROOT, under oracle/ref_shim.py;
+                        kind "reference") — or the torch port when it is not set (kind "port") — on the host cores
+
+Inputs and weights come from fixed seeds, so runs with the same arguments see identical inputs and two builds can be
+compared output for output through --dump-outputs.
 """
 import argparse
 import ctypes
@@ -36,7 +40,7 @@ METRIC = "forecast-windows/sec (B,N,W)=(32,358,12)"
 # BASELINE.json configs; B is per GPU (cfg4: global 128 on 4 GPUs, cfg5: global 256 on 8 GPUs)
 CONFIGS = {
     "cfg1": dict(B=32, N=140, W=12, H=3, gemm="auto",
-                 workload="ECG_data.csv N=140 W=12 H=3 batch=32 fp32 eval forward (BASELINE.json configs[0])"),
+                 workload="synthetic N=140 W=12 H=3 batch=32 fp32 eval forward (BASELINE.json configs[0] shape)"),
     "cfg2": dict(B=32, N=358, W=12, H=3, gemm="auto",
                  workload="synthetic N=358 W=12 H=3 batch=32 fp32 eval forward (BASELINE.json configs[1])"),
     "cfg3": dict(B=64, N=228, W=12, H=3, gemm="bf16",
@@ -129,23 +133,9 @@ class ClockSampler:
 
 
 def make_inputs(name, rank):
-    """(x (B,W,N), y (B,H,N), data tag).  cfg1 uses z-scored rows of the reference's ECG_data.csv when the staged
-    copy (baseline/_ref/dataset, shipped by oracle/fetch_reference.py) is present; everything else — and cfg1
-    without the CSV — uses the seeded synthetic generator of SURVEY.md §8(d)."""
-    import numpy as np
-    import torch
+    """(x (B,W,N), y (B,H,N), data tag): the seeded synthetic generator of SURVEY.md §8(d), seed 1234 + rank."""
     from stemgnn_b200 import synthetic
     c = CONFIGS[name]
-    if name == "cfg1":
-        for root in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-            csv = os.path.join(root, "dataset", "ECG_data.csv")
-            if os.path.isfile(csv):
-                data = np.loadtxt(csv, delimiter=",", dtype=np.float64)
-                data = (data - data.mean(axis=0)) / (data.std(axis=0) + 1e-12)       # z_score over the file
-                hi = [c["W"] + 97 * i + 13 * rank for i in range(c["B"])]            # B spread-out windows
-                x = np.stack([data[h - c["W"]:h] for h in hi]).astype(np.float32)
-                y = np.stack([data[h:h + c["H"]] for h in hi]).astype(np.float32)
-                return torch.from_numpy(x), torch.from_numpy(y), "ECG_data.csv rows (z-scored), reference dataset"
     x, y = synthetic.synthetic_batch(c["B"], c["N"], c["W"], c["H"], seed=1234 + rank)
     return x, y, "synthetic"
 
@@ -212,7 +202,7 @@ def run_ours(args, rank, world, local_rank):
     x_host = x_host.pin_memory()
     x_dev = x_host.to(dev)
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)      # > 126 MB L2
-    steps = args.steps if N <= 512 else max(3, min(args.steps, 10))    # cfg5: seconds per step
+    steps = args.steps
 
     def barrier():
         torch.cuda.synchronize()
@@ -229,17 +219,25 @@ def run_ours(args, rank, world, local_rank):
         model(x_dev)
         launches_per_forward = int(lib.stemgnn_launch_count() - c0)
         model.use_cuda_graph = True
-        for _ in range(max(args.warmup, 3)):
-            model(x_dev)
+        model(x_dev)                                  # captures the graph (synchronises the host) and uploads it
         # ---- device-timed: inputs resident in HBM, L2 flushed between steps -------------------
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
               for _ in range(steps)]
         sampler = ClockSampler(local_rank) if rank == 0 else None
         barrier()
+        # Every timed event pair must bracket device work only.  The stream is held for ~0.2 s by a spin kernel while the host
+        # enqueues the warm-up and timed steps (~0.2 ms of host time each; beyond the launch queue's depth the host is that
+        # queue ahead), and the warm-up runs back to back into the timed steps.  Otherwise a stall of the host thread
+        # (measured on a B200 at 1000 W: 8 and 70 ms, from NVML queries and the shared host CPUs), or the ~0.2 ms to submit the first
+        # step to an idle device, lands inside a timed step.
+        torch.cuda._sleep(400_000_000)                # cycles: 0.2 s at 2 GHz
+        for _ in range(max(args.warmup, 3)):
+            flush.zero_()
+            model(x_dev)
         for i in range(steps):
             flush.zero_()
             ev[i][0].record()
-            f_dev, _a = model(x_dev)
+            f_dev, a_dev = model(x_dev)
             ev[i][1].record()
         barrier()
         launches = launches_per_forward * steps      # + 3 torch copy kernels per step around the graph replay
@@ -338,6 +336,8 @@ def run_ours(args, rank, world, local_rank):
     dev_ms, e2e_ms, train_ms = float(t[0]), float(t[1]), float(t[2])
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, forecast=f_dev, attention=a_dev)
 
     peak_tf, peak_gbs, peak_src, extra_peaks = _peaks()
     gru_flops = 6.0 * B * N ** 3 + 12.0 * B * N * N               # SURVEY §8(d): recurrence + gates
@@ -429,6 +429,15 @@ def run_ours(args, rank, world, local_rank):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(out_dir, **arrays):
+    """What a caller of the timed forward receives — Model.forward's (forecast (B,H,N), attention (N,N)) — as
+    float32 <out_dir>/<name>.npy.  The largest configuration writes 17 MB (cfg5: attention 2048 x 2048)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def forward_flops(B, N, W, H, S=2, K=4):
     """SURVEY.md §8(d) dead-work-free forward flops."""
     T = MULTI * W
@@ -518,7 +527,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="cfg2", choices=sorted(CONFIGS))
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's forecast and attention (rank 0) to DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

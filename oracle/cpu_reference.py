@@ -1,12 +1,12 @@
 """TEST / BENCH INFRASTRUCTURE — not product code.
 
 The reference's own CPU implementation of the hot path, ready to call: the UNMODIFIED reference
-`models.base_model.Model` (mounted at /root/reference, or the staged byte-for-byte copy in
-git-ignored baseline/_ref/ — see oracle/fetch_reference.py) imported under the 4-patch shim of
-oracle/ref_shim.py, with the same seeded weights the CUDA model is loaded with.  When neither copy is
-present the torch port (oracle/torch_port.py, the same ATen op sequence) stands in and says so.
+`models.base_model.Model` (the checkout named by STEMGNN_REFERENCE_ROOT) imported under the 4-patch shim
+of oracle/ref_shim.py, with the same seeded weights the CUDA model is loaded with.  When it is not set the
+torch port (oracle/torch_port.py, the same ATen op sequence) stands in and says so.
 
-Only `bench.py` (`--impl reference`, `cpu_baseline`, the MAE-vs-ref parity figure) and `tests/` import this.
+Only `bench.py` (`--impl reference`, `cpu_baseline`, the MAE-vs-ref parity figure) and `oracle/make_golden.py`
+import this.
 """
 import os
 import time

@@ -1,9 +1,9 @@
 """TEST INFRASTRUCTURE — not product code.
 
-Loads the UNMODIFIED reference (microsoft/StemGNN): mounted read-only at /root/reference in the
-build container (where the golden vectors are minted), or the byte-for-byte staged copy in the
-git-ignored `baseline/_ref/` (oracle/fetch_reference.py) — the copy that travels to the GPU box,
-where `bench.py --impl reference`, `cpu_baseline` and the reference-vs-CUDA tests use it.
+Loads the UNMODIFIED reference (microsoft/StemGNN) from the checkout named by the environment variable
+STEMGNN_REFERENCE_ROOT.  `oracle/make_golden.py` mints `tests/golden/` from it; `bench.py --impl reference`
+and `cpu_baseline` use it when it is set and the torch port otherwise.  The tests never need it: what they
+compare against the reference is stored under `tests/golden/`.
 
 The reference pins torch==1.7.1 (requirements.txt:4) and uses four APIs that no longer
 exist on the container stack (torch 2.11 / numpy 2.3 / pandas 3.0).  They are patched
@@ -25,24 +25,11 @@ import importlib
 import os
 import sys
 
-_REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-
-def _find_reference_root():
-    """Mounted reference in the build container, else the byte-for-byte staged copy that
-    `oracle/fetch_reference.py` puts in git-ignored baseline/_ref/ (the only copy the GPU box has)."""
-    cands = [os.environ.get("STEMGNN_REFERENCE_ROOT"), "/root/reference", os.path.join(_REPO, "baseline", "_ref")]
-    for c in cands:
-        if c and os.path.isfile(os.path.join(c, "models", "base_model.py")):
-            return c
-    return cands[1]
-
-
-REFERENCE_ROOT = _find_reference_root()
+REFERENCE_ROOT = os.environ.get("STEMGNN_REFERENCE_ROOT", "")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "models", "base_model.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "models", "base_model.py"))
 
 
 def _install_patches():
@@ -95,7 +82,7 @@ def reference_modules():
     packages (not this repo's drop-in packages of the same names).  On exit the repo's own
     modules are restored in sys.modules."""
     if not reference_available():
-        raise RuntimeError(f"reference not found at {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference not found at {REFERENCE_ROOT!r} (set STEMGNN_REFERENCE_ROOT)")
     _install_patches()
     names = ("models", "data_loader", "utils")
     saved = {k: v for k, v in sys.modules.items()

@@ -2,7 +2,7 @@
 """Runs the UNMODIFIED reference `main.py` against this repo's drop-in `models/`, `data_loader/`,
 `utils/` packages (SURVEY.md §8(b) "Launching the unchanged main.py").
 
-    python run_main.py --device cuda:0 --epoch 1 [--dataset ECG_data ...]      # any main.py flag
+    STEMGNN_REFERENCE_ROOT=<checkout> python run_main.py --device cuda:0 --epoch 1 [--dataset ECG_data ...]   # any main.py flag
 
 `main.py` does `from models.handler import train, test`; run as a script it would import the
 reference's own packages, so this launcher puts the repo first on sys.path and executes the
@@ -17,21 +17,12 @@ import sys
 ROOT = os.path.dirname(os.path.abspath(__file__))
 
 
-def _reference_root():
-    """The mounted reference, else the staged byte-for-byte copy (git-ignored baseline/_ref/, see
-    oracle/fetch_reference.py) — the GPU box only has the latter."""
-    for c in (os.environ.get("STEMGNN_REFERENCE_ROOT"), "/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if c and os.path.isfile(os.path.join(c, "main.py")):
-            return c
-    return "/root/reference"
-
-
-REF = _reference_root()
+REF = os.environ.get("STEMGNN_REFERENCE_ROOT", "")       # a microsoft/StemGNN checkout
 
 
 def main():
     ref_main = os.path.join(REF, "main.py")
-    if not os.path.exists(ref_main):
+    if not REF or not os.path.exists(ref_main):
         raise SystemExit(f"reference main.py not found at {ref_main} (set STEMGNN_REFERENCE_ROOT)")
     work = os.environ.get("STEMGNN_WORKDIR", os.path.join(ROOT, "gpurun_out", "main_run"))
     os.makedirs(work, exist_ok=True)

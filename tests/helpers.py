@@ -35,6 +35,20 @@ def build_model(c, device, params=None):
     return m.to(device)
 
 
+def reference_default_init(N, W, H, multi, g):
+    """The reference Model's own default init (torch.manual_seed(0) before construction, main.py:52) as a state_dict.
+    The drop-in Model creates the same tensors in the same order, so it draws them; the per-tensor sums the reference's
+    init left in golden `g` (oracle/make_golden.py) confirm that they are the reference's."""
+    from models.base_model import Model
+    torch.manual_seed(0)
+    sd = {k: v.detach().clone() for k, v in Model(N, 2, W, multi, horizon=H).state_dict().items()}
+    assert sorted("init_sum." + k for k in sd) == sorted(f for f in g.files if f.startswith("init_sum."))
+    for k, v in sd.items():
+        a = v.double().numpy()
+        np.testing.assert_allclose([a.sum(), np.abs(a).sum()], g["init_sum." + k], rtol=1e-12, atol=0, err_msg=k)
+    return sd
+
+
 def assert_close(actual, expected, rtol=RTOL, atol=ATOL, msg=""):
     a = actual.detach().cpu().numpy() if torch.is_tensor(actual) else np.asarray(actual)
     e = expected.detach().cpu().numpy() if torch.is_tensor(expected) else np.asarray(expected)

@@ -7,7 +7,8 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import ref_shim, stemgnn_oracle as so, torch_port as tp
+from oracle import stemgnn_oracle as so, torch_port as tp
+from tests.helpers import reference_default_init
 
 RTOL, ATOL = 1e-3, 1e-4        # BASELINE.json north_star tolerance (fp32)
 TIGHT = dict(rtol=2e-4, atol=2e-5)
@@ -94,20 +95,18 @@ def test_param_shapes_and_count():
     assert abs(so.forward_flops(32, 358, 12, 3) / 1e9 - 28.3) < 0.2   # SURVEY.md §8(d)
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="reference tree not mounted")
-def test_oracle_against_live_reference_default_init():
-    """In the build container: reference Model at its OWN default init (torch.manual_seed(0),
-    main.py:52) vs both restatements — independent of the synthetic weights."""
-    m = ref_shim.build_reference_model(33, 12, 5, 3, seed=0)
-    m.eval()
-    sd = {k: v.detach().clone() for k, v in m.state_dict().items()}
+def test_oracle_against_live_reference_default_init(golden_dir):
+    """Reference Model at its OWN default init (torch.manual_seed(0), main.py:52) vs both restatements —
+    independent of the synthetic weights."""
+    g = np.load(os.path.join(golden_dir, "default_init_n33.npz"))
+    sd = reference_default_init(33, 12, 3, 5, g)
     assert {k: tuple(v.shape) for k, v in sd.items()} == tp.param_shapes(33, 12, 3)
     x, _ = tp.synthetic_batch(6, 33, 12, 3)
+    f_ref, a_ref = g["forecast"], g["attention"]
     with torch.no_grad():
-        f_ref, a_ref = m(x)
         f_port, a_port = tp.model_forward(x, sd)
     f_np, a_np = so.model_forward(x.numpy(), {k: v.numpy() for k, v in sd.items()})
-    np.testing.assert_allclose(f_port.numpy(), f_ref.numpy(), rtol=1e-5, atol=1e-6)
-    np.testing.assert_allclose(a_port.numpy(), a_ref.numpy(), rtol=1e-5, atol=1e-7)
-    np.testing.assert_allclose(f_np, f_ref.numpy(), **TIGHT)
-    np.testing.assert_allclose(a_np, a_ref.numpy(), **TIGHT)
+    np.testing.assert_allclose(f_port.numpy(), f_ref, rtol=1e-5, atol=1e-6)
+    np.testing.assert_allclose(a_port.numpy(), a_ref, rtol=1e-5, atol=1e-7)
+    np.testing.assert_allclose(f_np, f_ref, **TIGHT)
+    np.testing.assert_allclose(a_np, a_ref, **TIGHT)
