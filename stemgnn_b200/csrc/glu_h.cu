@@ -13,13 +13,11 @@
 // stream through a 3-stage TMA ring of 64-byte-row tiles (32 K columns per stage: SPLIT {W_hi, W_lo} of one side,
 // BF16 {W_left, W_right}); left / right accumulators side by side in TMEM, gate applied in the tcgen05.ld epilogue.
 // MMA issue: the whole warp runs the loop converged and one ELECTED lane issues (see gru_tc.cu for the measurement).
-#include <cuda.h>
-#include <cuda_bf16.h>
-#include <cuda_fp16.h>
 #include <stdlib.h>
 
 #include "common.cuh"
 #include "internal.cuh"
+#include "sm100.cuh"
 
 namespace sg {
 namespace {
@@ -32,111 +30,7 @@ constexpr int H_RIGHT_COL = 256;
 constexpr uint32_t H_TMEM_COLS = 512;
 constexpr int H_NSTG = 3;
 constexpr uint32_t H_A_CHUNK = H_BM * 128;       // 128 rows x 64 halves
-
-__device__ __forceinline__ uint32_t su32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-__device__ __forceinline__ void mb_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(su32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mb_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(su32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mb_wait(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = su32(bar);
-  uint32_t done = 0;
-  for (uint32_t spin = 0; !done; ++spin) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-    if (spin > (1u << 26)) __trap();
-  }
-}
-__device__ __forceinline__ void tma_2d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(su32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(su32(bar)), "r"(c0), "r"(c1)
-      : "memory");
-}
-// TMA load multicast to every CTA of `mask` (same CTA-relative smem offset and mbarrier in each)
-__device__ __forceinline__ void tma_2d_mc(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(su32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(su32(bar)), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_rank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tcf_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tcf_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ uint32_t elect1() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}" : "=r"(pred));
-  return pred;
-}
-__device__ __forceinline__ uint64_t desc_k(uint32_t smem_addr, uint32_t sbo, uint32_t layout) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr >> 4) & 0x3FFFu);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(sbo >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)layout << 61;          // 2 = SWIZZLE_128B, 4 = SWIZZLE_64B
-  return d;
-}
-// kind::f16: D fp32; A/B format 0 = fp16, 1 = bf16; K-major; M = 128
-__device__ __forceinline__ uint32_t idesc_h(int n, int bf16) {
-  return (1u << 4) | ((uint32_t)bf16 << 7) | ((uint32_t)bf16 << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(H_BM >> 4) << 24);
-}
-__device__ __forceinline__ void umma_h(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(acc)
-      : "memory");
-}
-__device__ __forceinline__ void commit_h(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(su32(bar)) : "memory");
-}
-__device__ __forceinline__ void commit_h_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(su32(bar)), "h"(mask)
-               : "memory");
-}
-__device__ __forceinline__ void ld16(uint32_t taddr, float (&v)[16]) {
-  uint32_t r[16];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-#pragma unroll
-  for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// fp32 -> 16-bit operand(s).  SPLIT: hi = fp16(sat(x)), lo = fp16(x - hi);  BF16: hi = bf16(x)
-template <bool SPLIT>
-__device__ __forceinline__ void to_h(float x, unsigned short& hi, unsigned short& lo) {
-  if (SPLIT) {
-    const float xs = fminf(fmaxf(x, -65504.f), 65504.f);
-    const __half h = __float2half_rn(xs);
-    hi = __half_as_ushort(h);
-    lo = __half_as_ushort(__float2half_rn(xs - __half2float(h)));
-  } else {
-    hi = __bfloat16_as_ushort(__float2bfloat16_rn(x));
-    lo = 0;
-  }
-}
+constexpr int H_SPIN_LOG2 = 26;                  // mbarrier polls before a lost arrival traps
 
 // ---- fp32 (rows x cols, ld) -> 16-bit hi / lo arrays (rows x ldh), zero padded columns --------------------------------
 template <bool SPLIT>
@@ -147,7 +41,7 @@ __global__ void split_rows_kernel(const float* __restrict__ src, int rows, int c
        idx += (long long)gridDim.x * blockDim.x) {
     const int r = (int)(idx / ldh), c = (int)(idx % ldh);
     unsigned short h = 0, l = 0;
-    if (c < cols) to_h<SPLIT>(src[(size_t)r * ld + c], h, l);
+    if (c < cols) split_f16_hi_lo(src[(size_t)r * ld + c], !SPLIT, h, l);
     hi[idx] = h;
     if (SPLIT) lo[idx] = l;
   }
@@ -174,9 +68,7 @@ struct GluHMaps {
 template <bool SPLIT, int CSZ>
 __global__ void __launch_bounds__(H_THREADS, 1) glu_chain_h_kernel(const __grid_constant__ GluHMaps maps, GluHArgs g) {
   extern __shared__ uint8_t smem_raw[];
-  // 1024-byte alignment by pointer arithmetic on the __shared__ array: an integer round trip would demote the epilogue's
-  // shared-memory accesses to generic LD/ST (seen in the ncu source view)
-  uint8_t* smem = smem_raw + ((1024u - (su32(smem_raw) & 1023u)) & 1023u);
+  uint8_t* smem = smem_raw + smem_pad1024(smem_raw);
   constexpr int NARR = SPLIT ? 2 : 1;
   const int N = g.N;
   const uint32_t w_bytes = (uint32_t)N * 64;            // N rows x 32 halves
@@ -203,54 +95,52 @@ __global__ void __launch_bounds__(H_THREADS, 1) glu_chain_h_kernel(const __grid_
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < H_NSTG; ++s) {
-      mb_init(&full_bar[s], 1);
-      mb_init(&empty_bar[s], CSZ);
+      mbarrier_init(&full_bar[s], 1);
+      mbarrier_init(&empty_bar[s], CSZ);
     }
-    mb_init(tmem_full_bar, 1);
-    mb_init(a_ready_bar, H_EPI);
-    mb_init(g_full_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbarrier_init(tmem_full_bar, 1);
+    mbarrier_init(a_ready_bar, H_EPI);
+    mbarrier_init(g_full_bar, 1);
+    fence_mbarrier_init();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(su32(tmem_slot)),
-                 "r"(H_TMEM_COLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tcgen05_alloc(tmem_slot, H_TMEM_COLS);
+    tcgen05_relinquish_alloc_permit();
   }
-  tcf_before();
+  tcgen05_fence_before();
   __syncthreads();
-  if (CSZ > 1) cluster_sync_all();      // the peer's barriers are initialised before any multicast lands
-  tcf_after();
+  if (CSZ > 1) cluster_sync();      // the peer's barriers are initialised before any multicast lands
+  tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  const uint32_t crank = CSZ > 1 ? cluster_rank() : 0u;
+  const uint32_t crank = CSZ > 1 ? cluster_ctarank() : 0u;
   constexpr uint16_t kMask = (uint16_t)((1u << CSZ) - 1u);
   const int wrows = N / CSZ;                                    // weight rows this CTA fetches per image
   const uint32_t woff = crank * (uint32_t)wrows * 64u;          //   and where they land inside an image of the stage
 
   if (warp == 0) {
     // ===== TMA producer (converged warp, elected lane): the input tile once, then the weight stages =====
-    if (elect1()) {
-      mb_expect_tx(g_full_bar, (uint32_t)(NARR * g_chunks) * H_A_CHUNK);
+    if (elect_one_sync()) {
+      mbarrier_arrive_expect_tx(g_full_bar, (uint32_t)(NARR * g_chunks) * H_A_CHUNK);
       for (int arr = 0; arr < NARR; ++arr)
         for (int c = 0; c < g_chunks; ++c)
-          tma_2d(a_buf + (size_t)(arr * 4 + c) * H_A_CHUNK, &maps.g[arr], g_full_bar, c * 64, m0);
+          tma_load_2d(a_buf + (size_t)(arr * 4 + c) * H_A_CHUNK, &maps.g[arr], g_full_bar, c * 64, m0);
       int it = 0;
       for (int l = 0; l < 3; ++l) {
         for (int kb = 0; kb < nkb[l]; ++kb) {
           for (int half = 0; half < (SPLIT ? 2 : 1); ++half, ++it) {     // SPLIT: stage = one side (left, then right)
             const int s = it % H_NSTG;
             const uint32_t ph = (uint32_t)(it / H_NSTG) & 1u;
-            mb_wait(&empty_bar[s], ph ^ 1u);
+            mbarrier_wait<H_SPIN_LOG2>(&empty_bar[s], ph ^ 1u);
             uint8_t* st = w_buf + (size_t)s * stage_bytes;
-            mb_expect_tx(&full_bar[s], stage_bytes);
+            mbarrier_arrive_expect_tx(&full_bar[s], stage_bytes);
             const CUtensorMap* m0p = SPLIT ? &maps.w[l][half][0] : &maps.w[l][0][0];
             const CUtensorMap* m1p = SPLIT ? &maps.w[l][half][1] : &maps.w[l][1][0];
             if (CSZ == 1) {
-              tma_2d(st, m0p, &full_bar[s], kb * 32, 0);
-              tma_2d(st + w_bytes, m1p, &full_bar[s], kb * 32, 0);
+              tma_load_2d(st, m0p, &full_bar[s], kb * 32, 0);
+              tma_load_2d(st + w_bytes, m1p, &full_bar[s], kb * 32, 0);
             } else {          // this CTA's share of the rows, delivered to every CTA of the pair
-              tma_2d_mc(st + woff, m0p, &full_bar[s], kb * 32, (int)crank * wrows, kMask);
-              tma_2d_mc(st + w_bytes + woff, m1p, &full_bar[s], kb * 32, (int)crank * wrows, kMask);
+              tma_load_2d_multicast(st + woff, m0p, &full_bar[s], kb * 32, (int)crank * wrows, kMask);
+              tma_load_2d_multicast(st + w_bytes + woff, m1p, &full_bar[s], kb * 32, (int)crank * wrows, kMask);
             }
           }
         }
@@ -259,50 +149,52 @@ __global__ void __launch_bounds__(H_THREADS, 1) glu_chain_h_kernel(const __grid_
     __syncwarp();
   } else if (warp == 1) {
     // ===== MMA issuer (converged warp, elected lane) =====
-    const uint32_t idesc = idesc_h(N, SPLIT ? 0 : 1);
-    const uint32_t a_addr = su32(a_buf);
-    mb_wait(g_full_bar, 0);
+    const uint32_t idesc = umma_idesc_m128(SPLIT ? UMMA_F16 : UMMA_BF16, N);
+    const uint32_t a_addr = smem_u32(a_buf);
+    mbarrier_wait<H_SPIN_LOG2>(g_full_bar, 0);
     int it = 0;
     for (int l = 0; l < 3; ++l) {
       if (l > 0) {
-        mb_wait(a_ready_bar, (uint32_t)(l - 1) & 1u);
-        tcf_after();
+        mbarrier_wait<H_SPIN_LOG2>(a_ready_bar, (uint32_t)(l - 1) & 1u);
+        tcgen05_fence_after();
       }
       for (int kb = 0; kb < nkb[l]; ++kb) {
         for (int half = 0; half < (SPLIT ? 2 : 1); ++half, ++it) {
           const int s = it % H_NSTG;
           const uint32_t ph = (uint32_t)(it / H_NSTG) & 1u;
-          mb_wait(&full_bar[s], ph);
-          tcf_after();
-          if (elect1()) {
-            const uint32_t w0 = su32(w_buf + (size_t)s * stage_bytes), w1 = w0 + w_bytes;
+          mbarrier_wait<H_SPIN_LOG2>(&full_bar[s], ph);
+          tcgen05_fence_after();
+          if (elect_one_sync()) {
+            const uint32_t w0 = smem_u32(w_buf + (size_t)s * stage_bytes), w1 = w0 + w_bytes;
 #pragma unroll
             for (int kk = 0; kk < 2; ++kk) {
               const int k16 = kb * 2 + kk;
               if (k16 < nk16[l]) {
                 const uint32_t a_off = (uint32_t)(k16 >> 2) * H_A_CHUNK + (uint32_t)(k16 & 3) * 32u;
-                const uint64_t a_hi = desc_k(a_addr + a_off, 1024, 2);
+                const uint64_t a_hi = umma_desc_kmajor(a_addr + a_off, 1024, UMMA_SWIZZLE_128B);
                 const uint32_t acc = k16 > 0 ? 1u : 0u;
                 if (SPLIT) {
-                  const uint64_t a_lo = desc_k(a_addr + 4 * H_A_CHUNK + a_off, 1024, 2);
+                  const uint64_t a_lo = umma_desc_kmajor(a_addr + 4 * H_A_CHUNK + a_off, 1024, UMMA_SWIZZLE_128B);
                   const uint32_t d = tmem_base + (half ? H_RIGHT_COL : 0);
-                  const uint64_t b_hi = desc_k(w0 + kk * 32, 512, 4), b_lo = desc_k(w1 + kk * 32, 512, 4);
-                  umma_h(d, a_hi, b_hi, idesc, acc);
-                  umma_h(d, a_hi, b_lo, idesc, 1u);
-                  umma_h(d, a_lo, b_hi, idesc, 1u);
+                  const uint64_t b_hi = umma_desc_kmajor(w0 + kk * 32, 512, UMMA_SWIZZLE_64B);
+                  const uint64_t b_lo = umma_desc_kmajor(w1 + kk * 32, 512, UMMA_SWIZZLE_64B);
+                  tcgen05_mma_f16(d, a_hi, b_hi, idesc, acc);
+                  tcgen05_mma_f16(d, a_hi, b_lo, idesc, 1u);
+                  tcgen05_mma_f16(d, a_lo, b_hi, idesc, 1u);
                 } else {
-                  umma_h(tmem_base, a_hi, desc_k(w0 + kk * 32, 512, 4), idesc, acc);
-                  umma_h(tmem_base + H_RIGHT_COL, a_hi, desc_k(w1 + kk * 32, 512, 4), idesc, acc);
+                  tcgen05_mma_f16(tmem_base, a_hi, umma_desc_kmajor(w0 + kk * 32, 512, UMMA_SWIZZLE_64B), idesc, acc);
+                  tcgen05_mma_f16(tmem_base + H_RIGHT_COL, a_hi, umma_desc_kmajor(w1 + kk * 32, 512, UMMA_SWIZZLE_64B), idesc,
+                                  acc);
                 }
               }
             }
-            if (CSZ == 1) commit_h(&empty_bar[s]);
-            else commit_h_mc(&empty_bar[s], kMask);     // signalled in every CTA that multicasts into this stage
+            if (CSZ == 1) tcgen05_commit(&empty_bar[s]);
+            else tcgen05_commit_multicast(&empty_bar[s], kMask);     // signalled in every CTA that multicasts into this stage
           }
           __syncwarp();
         }
       }
-      if (elect1()) commit_h(tmem_full_bar);
+      if (elect_one_sync()) tcgen05_commit(tmem_full_bar);
       __syncwarp();
     }
   } else {
@@ -312,7 +204,7 @@ __global__ void __launch_bounds__(H_THREADS, 1) glu_chain_h_kernel(const __grid_
       s_bias[(l * 2 + 0) * N + c] = __ldg(g.bl[l] + c);
       s_bias[(l * 2 + 1) * N + c] = __ldg(g.br[l] + c);
     }
-    asm volatile("bar.sync 1, 256;" ::: "memory");
+    bar_sync<1, 256>();
     const int quarter = warp & 3;
     const int half = (warp - 2) >> 2;                      // column half of this warp
     const int c_split = ((N / 16 + 1) / 2) * 16;
@@ -321,21 +213,21 @@ __global__ void __launch_bounds__(H_THREADS, 1) glu_chain_h_kernel(const __grid_
     const int row = m0 + rloc;
     const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16);
     for (int l = 0; l < 3; ++l) {
-      mb_wait(tmem_full_bar, (uint32_t)l & 1u);
-      tcf_after();
+      mbarrier_wait<H_SPIN_LOG2>(tmem_full_bar, (uint32_t)l & 1u);
+      tcgen05_fence_after();
       const float* sbl = s_bias + (l * 2 + 0) * N;
       const float* sbr = s_bias + (l * 2 + 1) * N;
       float* gout = l == 2 ? g.out3 : g.act[l];
       const int ldo = l == 2 ? g.ldo3 : N;
       for (int c = c_begin; c < c_end; c += 16) {
         float lv[16], rv[16], o[16];
-        ld16(taddr + c, lv);
-        ld16(taddr + H_RIGHT_COL + c, rv);
-        ld_wait();
+        tcgen05_ld_32x32b_x16(taddr + c, lv);
+        tcgen05_ld_32x32b_x16(taddr + H_RIGHT_COL + c, rv);
+        tcgen05_wait_ld();
 #pragma unroll
         for (int j = 0; j < 16; ++j) {
           lv[j] += sbl[c + j];
-          rv[j] = __fdividef(1.0f, 1.0f + __expf(-(rv[j] + sbr[c + j])));
+          rv[j] = fast_sigmoid(rv[j] + sbr[c + j]);
           o[j] = lv[j] * rv[j];
         }
         if (l < 2) {   // next layer's A operand: 64-half chunks, rows of 128 bytes, 16-byte granules XOR-swizzled by row % 8
@@ -343,8 +235,8 @@ __global__ void __launch_bounds__(H_THREADS, 1) glu_chain_h_kernel(const __grid_
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
             unsigned short h0, l0, h1, l1;
-            to_h<SPLIT>(o[2 * j], h0, l0);
-            to_h<SPLIT>(o[2 * j + 1], h1, l1);
+            split_f16_hi_lo(o[2 * j], !SPLIT, h0, l0);
+            split_f16_hi_lo(o[2 * j + 1], !SPLIT, h1, l1);
             hp[j] = (uint32_t)h0 | ((uint32_t)h1 << 16);
             lp[j] = (uint32_t)l0 | ((uint32_t)l1 << 16);
           }
@@ -378,50 +270,19 @@ __global__ void __launch_bounds__(H_THREADS, 1) glu_chain_h_kernel(const __grid_
       }
       if (l < 2) {
         // K padding of the next A tile (columns N .. round16(N)) must be finite zeros: N % 16 == 0 is required by the host
-        tcf_before();
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(su32(a_ready_bar)) : "memory");
+        tcgen05_fence_before();
+        fence_proxy_async_shared();
+        mbarrier_arrive(a_ready_bar);
       }
     }
   }
-  tcf_before();
+  tcgen05_fence_before();
   __syncthreads();
   if (warp == 1) {
-    tcf_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(H_TMEM_COLS) : "memory");
+    tcgen05_fence_after();
+    tcgen05_dealloc(tmem_base, H_TMEM_COLS);
   }
-  if (CSZ > 1) cluster_sync_all();      // no CTA exits while its peer can still signal its barriers
-}
-
-typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                             const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                             CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeFn encode_fn() {
-  static EncodeFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeFn>(p);
-    else
-      (void)cudaGetLastError();
-  }
-  return fn;
-}
-// 2-D 16-bit tensor (rows x cols, row stride ldh elements); box = box_rows x box_cols
-bool map_h(EncodeFn enc, CUtensorMap* map, const void* base, int rows, int cols, int ldh, int box_rows, int box_cols,
-           bool bf16) {
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)ldh * 2};
-  cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  return enc(map, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base),
-             dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             box_cols == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+  if (CSZ > 1) cluster_sync();      // no CTA exits while its peer can still signal its barriers
 }
 
 }  // namespace
@@ -442,8 +303,6 @@ int glu_chain_h(int mode, int M, int N, int K1, const float* G, int ldg, const f
                 cudaStream_t st, int g_ready) {
   if (N % 16 != 0 || N < 16 || N > 256 || K1 < 1 || K1 > 256 || (ldo3 & 3) != 0 || scratch == nullptr) return -1;
   if ((reinterpret_cast<uintptr_t>(scratch) & 15) || (reinterpret_cast<uintptr_t>(out3) & 15)) return -1;
-  EncodeFn enc = encode_fn();
-  if (enc == nullptr) return -1;
   const bool split = mode == 0;
   const int k1p = (K1 + 63) / 64 * 64;
   // scratch layout (16-bit elements): G_hi, G_lo (M x k1p) | per layer, side: W_hi, W_lo (N x Kp)
@@ -458,6 +317,23 @@ int glu_chain_h(int mode, int M, int N, int K1, const float* G, int ldg, const f
         w_img[l][sd][arr] = wp;
         wp += (size_t)N * kp[l];
       }
+  // CTA pairs with multicast weight stages unless disabled (STEMGNN_GLU_NO_MULTICAST) or half an image breaks the 8-row atom
+  static const bool no_mc = getenv("STEMGNN_GLU_NO_MULTICAST") != nullptr;
+  const int csz = (!no_mc && N % 16 == 0) ? 2 : 1;
+  // the maps come first: nothing is enqueued when the tensor maps cannot be made
+  GluHMaps maps;
+  const CUtensorMapDataType dt = split ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+  // logical width K1, pitch k1p: the TMA unit zero-fills columns K1 .. k1p, so producers of the images (the tcgen05 graph
+  // Fourier transform's epilogue) need not write the padding
+  if (!make_tensor_map_2d(&maps.g[0], dt, g_hi, M, K1, k1p * 2ull, H_BM, 64, CU_TENSOR_MAP_SWIZZLE_128B) ||
+      !make_tensor_map_2d(&maps.g[1], dt, g_lo, M, K1, k1p * 2ull, H_BM, 64, CU_TENSOR_MAP_SWIZZLE_128B))
+    return -1;
+  for (int l = 0; l < 3; ++l)
+    for (int sd = 0; sd < 2; ++sd)
+      for (int arr = 0; arr < 2; ++arr)
+        if (!make_tensor_map_2d(&maps.w[l][sd][arr], dt, w_img[l][sd][arr], N, kp[l], kp[l] * 2ull, N / csz, 32,
+                                CU_TENSOR_MAP_SWIZZLE_64B))
+          return -1;
   auto conv = [&](const float* src, int rows, int cols, int ld, unsigned short* hi, unsigned short* lo, int ldh) -> int {
     const long long total = (long long)rows * ldh;
     const int blocks = (int)((total + 255) / 256 < 148 * 16 ? (total + 255) / 256 : 148 * 16);
@@ -471,19 +347,6 @@ int glu_chain_h(int mode, int M, int N, int K1, const float* G, int ldg, const f
     for (int l = 0; l < 3; ++l)
       for (int sd = 0; sd < 2; ++sd)
         SG_TRY(conv(w[l][sd], N, l == 0 ? K1 : N, l == 0 ? K1 : N, w_img[l][sd][0], w_img[l][sd][1], kp[l]));
-  // CTA pairs with multicast weight stages unless disabled (STEMGNN_GLU_NO_MULTICAST) or half an image breaks the 8-row atom
-  static const bool no_mc = getenv("STEMGNN_GLU_NO_MULTICAST") != nullptr;
-  const int csz = (!no_mc && N % 16 == 0) ? 2 : 1;
-  GluHMaps maps;
-  const bool bf = !split;
-  // logical width K1, pitch k1p: the TMA unit zero-fills columns K1 .. k1p, so producers of the images (the tcgen05 graph
-  // Fourier transform's epilogue) need not write the padding
-  if (!map_h(enc, &maps.g[0], g_hi, M, K1, k1p, H_BM, 64, bf) || !map_h(enc, &maps.g[1], g_lo, M, K1, k1p, H_BM, 64, bf))
-    return -1;
-  for (int l = 0; l < 3; ++l)
-    for (int sd = 0; sd < 2; ++sd)
-      for (int arr = 0; arr < 2; ++arr)
-        if (!map_h(enc, &maps.w[l][sd][arr], w_img[l][sd][arr], N, kp[l], kp[l], N / csz, 32, bf)) return -1;
   const size_t smem = (size_t)(split ? 2 : 1) * 4 * H_A_CHUNK + (size_t)H_NSTG * 2 * N * 64 + 128 +
                       (size_t)6 * N * sizeof(float) + 1024;
   if (smem > 227 * 1024) return -1;

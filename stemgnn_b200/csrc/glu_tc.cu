@@ -15,11 +15,11 @@
 //
 // Operand precision: fp32 bit patterns are fed directly; kind::tf32 reads the top 19 bits
 // (truncation).  Error budget vs the fp32 reference: DESIGN.md "Precision".
-#include <cuda.h>
 #include <stdlib.h>
 
 #include "common.cuh"
 #include "internal.cuh"
+#include "sm100.cuh"
 
 namespace sg {
 
@@ -31,110 +31,7 @@ constexpr int TC_STAGES = 2;
 constexpr int TC_THREADS = 192;
 constexpr int TC_RIGHT_COL = 256;     // TMEM column of the right accumulator
 constexpr uint32_t TC_TMEM_COLS = 512;
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) {
-  return static_cast<uint32_t>(__cvta_generic_to_shared(p));
-}
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = smem_u32(bar);
-  uint32_t done = 0;
-  for (uint32_t spin = 0; !done; ++spin) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-    if (spin > (1u << 26)) __trap();   // bring-up guard: a lost arrival must fail, not hang the GPU
-  }
-}
-__device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-      : "memory");
-}
-// TMA load multicast to every CTA of `mask` (same CTA-relative smem offset and mbarrier in each)
-__device__ __forceinline__ void tma_load_2d_mc(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1,
-                                               uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"(mask)
-               : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-// K-major, 128B-swizzled operand tile: rows of 128 bytes, 8-row groups 1024 bytes apart.
-// Same for 64-byte rows (16 fp32 along K per stage): SWIZZLE_64B, 8-row groups 512 bytes apart.
-__device__ __forceinline__ uint64_t umma_desc_sw64(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr >> 4) & 0x3FFFu);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(512 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)4 << 61;                             // layout type SWIZZLE_64B
-  return d;
-}
-__device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr >> 4) & 0x3FFFu);        // start address            bits [0,14)
-  d |= (uint64_t)1 << 16;                             // leading byte offset (unused for swizzled K-major)
-  d |= (uint64_t)(1024 >> 4) << 32;                   // stride byte offset = 1024 bits [32,46)
-  d |= (uint64_t)1 << 46;                             // descriptor version (sm_100)
-  d |= (uint64_t)2 << 61;                             // layout type SWIZZLE_128B
-  return d;
-}
-// kind::tf32, fp32 accumulate, A and B K-major, M=128
-__device__ __forceinline__ uint32_t umma_idesc_tf32(int n) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
-}
-__device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
-                                          uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
-  uint32_t r[16];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-#pragma unroll
-  for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+constexpr int TC_SPIN_LOG2 = 26;      // mbarrier polls before a lost arrival traps
 
 struct GluTcArgs {
   const float* bl; const float* br;
@@ -154,10 +51,12 @@ glu_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__
               const __grid_constant__ CUtensorMap map_wr, GluTcArgs g) {
   extern __shared__ uint8_t smem_raw[];
   // 1024-byte alignment is required by the 128B swizzle pattern
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // keeps the shared address space (LDS/STS)
+  uint8_t* smem = smem_raw + smem_pad1024(smem_raw);
   const int N = g.N;
   constexpr int RB = BK * 4;                        // bytes per tile row
   constexpr int NSTAGE = BK == 32 ? 2 : 5;
+  constexpr UmmaSwizzle SWIZZLE = BK == 32 ? UMMA_SWIZZLE_128B : UMMA_SWIZZLE_64B;
+  constexpr uint32_t SBO = 8 * RB;                  // 8-row groups of the swizzled tiles
   const uint32_t a_bytes = TC_BM * RB, w_bytes = (uint32_t)N * RB;
   const uint32_t stage_bytes = a_bytes + 2 * w_bytes;
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + NSTAGE * stage_bytes);
@@ -175,25 +74,23 @@ glu_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__
   constexpr uint16_t kMask = (uint16_t)((1u << CSZ) - 1u);
   if (threadIdx.x == 0) {
     for (int s = 0; s < NSTAGE; ++s) {
-      mbar_init(&full_bar[s], 1);
-      mbar_init(&empty_bar[s], CSZ);       // a stage is free once EVERY CTA of the cluster has consumed it
+      mbarrier_init(&full_bar[s], 1);
+      mbarrier_init(&empty_bar[s], CSZ);       // a stage is free once EVERY CTA of the cluster has consumed it
     }
-    mbar_init(tmem_full_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&map_a)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&map_wl)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&map_wr)) : "memory");
+    mbarrier_init(tmem_full_bar, 1);
+    fence_mbarrier_init();
+    prefetch_tensormap(&map_a);
+    prefetch_tensormap(&map_wl);
+    prefetch_tensormap(&map_wr);
   }
   if (warp == 1) {   // the allocating warp also owns the dealloc
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(TC_TMEM_COLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tcgen05_alloc(tmem_slot, TC_TMEM_COLS);
+    tcgen05_relinquish_alloc_permit();
   }
-  tc_fence_before();
+  tcgen05_fence_before();
   __syncthreads();
-  if (CSZ > 1) cluster_sync_all();   // peer barriers are initialised before any multicast lands
-  tc_fence_after();
+  if (CSZ > 1) cluster_sync();   // peer barriers are initialised before any multicast lands
+  tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0) {
@@ -201,9 +98,9 @@ glu_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__
       for (int kb = 0; kb < num_kb; ++kb) {
         const int s = kb % NSTAGE;
         const uint32_t ph = (uint32_t)(kb / NSTAGE) & 1u;
-        mbar_wait(&empty_bar[s], ph ^ 1u);
+        mbarrier_wait<TC_SPIN_LOG2>(&empty_bar[s], ph ^ 1u);
         uint8_t* st = smem + (size_t)s * stage_bytes;
-        mbar_arrive_expect_tx(&full_bar[s], stage_bytes);
+        mbarrier_arrive_expect_tx(&full_bar[s], stage_bytes);
         tma_load_2d(st, &map_a, &full_bar[s], kb * BK, m0);
         if (CSZ == 1) {
           tma_load_2d(st + a_bytes, &map_wl, &full_bar[s], kb * BK, 0);
@@ -211,57 +108,57 @@ glu_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__
         } else {         // this CTA's share of the weight rows, delivered to every CTA of the cluster
           const int rows = N / CSZ;
           const uint32_t off = crank * (uint32_t)rows * (uint32_t)RB;
-          tma_load_2d_mc(st + a_bytes + off, &map_wl, &full_bar[s], kb * BK, (int)crank * rows, kMask);
-          tma_load_2d_mc(st + a_bytes + w_bytes + off, &map_wr, &full_bar[s], kb * BK, (int)crank * rows, kMask);
+          tma_load_2d_multicast(st + a_bytes + off, &map_wl, &full_bar[s], kb * BK, (int)crank * rows, kMask);
+          tma_load_2d_multicast(st + a_bytes + w_bytes + off, &map_wr, &full_bar[s], kb * BK, (int)crank * rows, kMask);
         }
       }
     }
   } else if (warp == 1) {
     if (lane == 0) {   // ===== MMA issuer =====
-      const uint32_t idesc = umma_idesc_tf32(N);
+      const uint32_t idesc = umma_idesc_m128(UMMA_TF32, N);
       for (int kb = 0; kb < num_kb; ++kb) {
         const int s = kb % NSTAGE;
         const uint32_t ph = (uint32_t)(kb / NSTAGE) & 1u;
-        mbar_wait(&full_bar[s], ph);
-        tc_fence_after();
+        mbarrier_wait<TC_SPIN_LOG2>(&full_bar[s], ph);
+        tcgen05_fence_after();
         const uint32_t a_addr = smem_u32(smem + (size_t)s * stage_bytes);
         const uint32_t wl_addr = a_addr + a_bytes, wr_addr = wl_addr + w_bytes;
 #pragma unroll
         for (int kk = 0; kk < BK / 8; ++kk) {   // 8 tf32 = 32 bytes along K per instruction
-          const uint64_t ad = BK == 32 ? umma_desc_sw128(a_addr + kk * 32) : umma_desc_sw64(a_addr + kk * 32);
+          const uint64_t ad = umma_desc_kmajor(a_addr + kk * 32, SBO, SWIZZLE);
           const uint32_t acc = (kb > 0 || kk > 0) ? 1u : 0u;
-          const uint64_t dl = BK == 32 ? umma_desc_sw128(wl_addr + kk * 32) : umma_desc_sw64(wl_addr + kk * 32);
-          const uint64_t dr = BK == 32 ? umma_desc_sw128(wr_addr + kk * 32) : umma_desc_sw64(wr_addr + kk * 32);
-          umma_tf32(tmem_base, ad, dl, idesc, acc);
-          umma_tf32(tmem_base + TC_RIGHT_COL, ad, dr, idesc, acc);
+          const uint64_t dl = umma_desc_kmajor(wl_addr + kk * 32, SBO, SWIZZLE);
+          const uint64_t dr = umma_desc_kmajor(wr_addr + kk * 32, SBO, SWIZZLE);
+          tcgen05_mma_tf32(tmem_base, ad, dl, idesc, acc);
+          tcgen05_mma_tf32(tmem_base + TC_RIGHT_COL, ad, dr, idesc, acc);
         }
-        if (CSZ == 1) umma_commit(&empty_bar[s]);   // stage reusable once these MMAs have read it
-        else umma_commit_mc(&empty_bar[s], kMask);  //   (signalled in every CTA that multicasts into it)
+        if (CSZ == 1) tcgen05_commit(&empty_bar[s]);   // stage reusable once these MMAs have read it
+        else tcgen05_commit_multicast(&empty_bar[s], kMask);  //   (signalled in every CTA that multicasts into it)
       }
-      umma_commit(tmem_full_bar);                   // accumulators complete
+      tcgen05_commit(tmem_full_bar);                   // accumulators complete
     }
   } else {             // ===== epilogue: warps 2..5 =====
     for (int i = threadIdx.x - 64; i < N; i += 128) {        // overlaps with the MMA main loop
       s_bl[i] = __ldg(g.bl + i);
       s_br[i] = __ldg(g.br + i);
     }
-    asm volatile("bar.sync 1, 128;" ::: "memory");           // epilogue warps only
-    mbar_wait(tmem_full_bar, 0);
-    tc_fence_after();
+    bar_sync<1, 128>();           // epilogue warps only
+    mbarrier_wait<TC_SPIN_LOG2>(tmem_full_bar, 0);
+    tcgen05_fence_after();
     const int quarter = warp & 3;                   // TMEM lane quarter this warp may read
     const int row = m0 + quarter * 32 + lane;
     const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16);
     for (int c = 0; c < N; c += 16) {
       float l[16], r[16];
-      tmem_ld16(taddr + c, l);
-      tmem_ld16(taddr + TC_RIGHT_COL + c, r);
-      tmem_ld_wait();
+      tcgen05_ld_32x32b_x16(taddr + c, l);
+      tcgen05_ld_32x32b_x16(taddr + TC_RIGHT_COL + c, r);
+      tcgen05_wait_ld();
       if (row < g.M) {
         float o[16];
 #pragma unroll
         for (int j = 0; j < 16; ++j) {
           l[j] += s_bl[c + j];
-          r[j] = __fdividef(1.0f, 1.0f + __expf(-(r[j] + s_br[c + j])));
+          r[j] = fast_sigmoid(r[j] + s_br[c + j]);
           o[j] = l[j] * r[j];
         }
         float4* po = reinterpret_cast<float4*>(g.out + (size_t)row * g.ldo + c);
@@ -279,12 +176,11 @@ glu_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__
       }
     }
   }
-  tc_fence_before();
+  tcgen05_fence_before();
   __syncthreads();
   if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TC_TMEM_COLS)
-                 : "memory");
+    tcgen05_fence_after();
+    tcgen05_dealloc(tmem_base, TC_TMEM_COLS);
   }
 }
 
@@ -308,7 +204,7 @@ glu_chain_tc_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_cons
                     const __grid_constant__ CUtensorMap map_w2r, const __grid_constant__ CUtensorMap map_w3l,
                     const __grid_constant__ CUtensorMap map_w3r, GluChainArgs g) {
   extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // keeps the shared address space (LDS/STS)
+  uint8_t* smem = smem_raw + smem_pad1024(smem_raw);
   constexpr int NSTG = 3;
   constexpr uint32_t A_CHUNK = TC_BM * 128;            // 128 rows x 32 fp32
   const int N = g.N;
@@ -334,37 +230,35 @@ glu_chain_tc_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_cons
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < NSTG; ++s) {
-      mbar_init(&full_bar[s], 1);
-      mbar_init(&empty_bar[s], 1);
+      mbarrier_init(&full_bar[s], 1);
+      mbarrier_init(&empty_bar[s], 1);
     }
-    mbar_init(tmem_full_bar, 1);
-    mbar_init(a_ready_bar, 128);
-    mbar_init(g_full_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbarrier_init(tmem_full_bar, 1);
+    mbarrier_init(a_ready_bar, 128);
+    mbarrier_init(g_full_bar, 1);
+    fence_mbarrier_init();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(TC_TMEM_COLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tcgen05_alloc(tmem_slot, TC_TMEM_COLS);
+    tcgen05_relinquish_alloc_permit();
   }
-  tc_fence_before();
+  tcgen05_fence_before();
   __syncthreads();
-  tc_fence_after();
+  tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0) {
     if (lane == 0) {   // ===== TMA producer: the input tile once, then the weights of the three layers =====
-      mbar_arrive_expect_tx(g_full_bar, (uint32_t)g_chunks * A_CHUNK);
+      mbarrier_arrive_expect_tx(g_full_bar, (uint32_t)g_chunks * A_CHUNK);
       for (int c = 0; c < g_chunks; ++c) tma_load_2d(a_buf + (size_t)c * A_CHUNK, &map_g, g_full_bar, c * 32, m0);
       int it = 0;
       for (int l = 0; l < 3; ++l) {
         for (int kb = 0; kb < nkb[l]; ++kb, ++it) {
           const int s = it % NSTG;
           const uint32_t ph = (uint32_t)(it / NSTG) & 1u;
-          mbar_wait(&empty_bar[s], ph ^ 1u);
+          mbarrier_wait<TC_SPIN_LOG2>(&empty_bar[s], ph ^ 1u);
           uint8_t* st = w_buf + (size_t)s * stage_bytes;
-          mbar_arrive_expect_tx(&full_bar[s], stage_bytes);
+          mbarrier_arrive_expect_tx(&full_bar[s], stage_bytes);
           tma_load_2d(st, wmaps[l][0], &full_bar[s], kb * 16, 0);
           tma_load_2d(st + w_bytes, wmaps[l][1], &full_bar[s], kb * 16, 0);
         }
@@ -372,32 +266,34 @@ glu_chain_tc_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_cons
     }
   } else if (warp == 1) {
     if (lane == 0) {   // ===== MMA issuer =====
-      const uint32_t idesc = umma_idesc_tf32(N);
+      const uint32_t idesc = umma_idesc_m128(UMMA_TF32, N);
       const uint32_t a_addr = smem_u32(a_buf);
-      mbar_wait(g_full_bar, 0);
+      mbarrier_wait<TC_SPIN_LOG2>(g_full_bar, 0);
       int it = 0;
       for (int l = 0; l < 3; ++l) {
         if (l > 0) {                       // A tile of this layer written by the epilogue, TMEM free again
-          mbar_wait(a_ready_bar, (uint32_t)(l - 1) & 1u);
-          tc_fence_after();
+          mbarrier_wait<TC_SPIN_LOG2>(a_ready_bar, (uint32_t)(l - 1) & 1u);
+          tcgen05_fence_after();
         }
         for (int kb = 0; kb < nkb[l]; ++kb, ++it) {
           const int s = it % NSTG;
           const uint32_t ph = (uint32_t)(it / NSTG) & 1u;
-          mbar_wait(&full_bar[s], ph);
-          tc_fence_after();
+          mbarrier_wait<TC_SPIN_LOG2>(&full_bar[s], ph);
+          tcgen05_fence_after();
           const uint32_t wl_addr = smem_u32(w_buf + (size_t)s * stage_bytes), wr_addr = wl_addr + w_bytes;
 #pragma unroll
           for (int kk = 0; kk < 2; ++kk) {
             const int k0 = kb * 16 + kk * 8;
-            const uint64_t ad = umma_desc_sw128(a_addr + (uint32_t)(k0 >> 5) * A_CHUNK + (uint32_t)(k0 & 31) * 4);
+            const uint64_t ad =
+                umma_desc_kmajor(a_addr + (uint32_t)(k0 >> 5) * A_CHUNK + (uint32_t)(k0 & 31) * 4, 1024, UMMA_SWIZZLE_128B);
             const uint32_t acc = (kb > 0 || kk > 0) ? 1u : 0u;
-            umma_tf32(tmem_base, ad, umma_desc_sw64(wl_addr + kk * 32), idesc, acc);
-            umma_tf32(tmem_base + TC_RIGHT_COL, ad, umma_desc_sw64(wr_addr + kk * 32), idesc, acc);
+            tcgen05_mma_tf32(tmem_base, ad, umma_desc_kmajor(wl_addr + kk * 32, 512, UMMA_SWIZZLE_64B), idesc, acc);
+            tcgen05_mma_tf32(tmem_base + TC_RIGHT_COL, ad, umma_desc_kmajor(wr_addr + kk * 32, 512, UMMA_SWIZZLE_64B), idesc,
+                             acc);
           }
-          umma_commit(&empty_bar[s]);
+          tcgen05_commit(&empty_bar[s]);
         }
-        umma_commit(tmem_full_bar);
+        tcgen05_commit(tmem_full_bar);
       }
     }
   } else {             // ===== epilogue: warps 2..5 =====
@@ -406,27 +302,27 @@ glu_chain_tc_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_cons
       s_bias[(l * 2 + 0) * N + c] = __ldg(g.bl[l] + c);
       s_bias[(l * 2 + 1) * N + c] = __ldg(g.br[l] + c);
     }
-    asm volatile("bar.sync 1, 128;" ::: "memory");
+    bar_sync<1, 128>();
     const int quarter = warp & 3;
     const int rloc = quarter * 32 + lane;               // row inside the tile = TMEM lane
     const int row = m0 + rloc;
     const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16);
     for (int l = 0; l < 3; ++l) {
-      mbar_wait(tmem_full_bar, (uint32_t)l & 1u);
-      tc_fence_after();
+      mbarrier_wait<TC_SPIN_LOG2>(tmem_full_bar, (uint32_t)l & 1u);
+      tcgen05_fence_after();
       const float* sbl = s_bias + (l * 2 + 0) * N;
       const float* sbr = s_bias + (l * 2 + 1) * N;
       float* gout = l == 2 ? g.out3 : g.act[l];
       const int ldo = l == 2 ? g.ldo3 : N;
       for (int c = 0; c < N; c += 16) {
         float lv[16], rv[16], o[16];
-        tmem_ld16(taddr + c, lv);
-        tmem_ld16(taddr + TC_RIGHT_COL + c, rv);
-        tmem_ld_wait();
+        tcgen05_ld_32x32b_x16(taddr + c, lv);
+        tcgen05_ld_32x32b_x16(taddr + TC_RIGHT_COL + c, rv);
+        tcgen05_wait_ld();
 #pragma unroll
         for (int j = 0; j < 16; ++j) {
           lv[j] += sbl[c + j];
-          rv[j] = __fdividef(1.0f, 1.0f + __expf(-(rv[j] + sbr[c + j])));
+          rv[j] = fast_sigmoid(rv[j] + sbr[c + j]);
           o[j] = lv[j] * rv[j];
         }
         if (l < 2) {   // next layer's A operand: K-major rows of 128 bytes, 16-byte chunks XOR-swizzled by row%8
@@ -455,18 +351,17 @@ glu_chain_tc_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_cons
         }
       }
       if (l < 2) {
-        tc_fence_before();                                               // TMEM reads done before the next MMAs
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // generic-proxy smem writes -> tensor core
-        asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(a_ready_bar)) : "memory");
+        tcgen05_fence_before();                                               // TMEM reads done before the next MMAs
+        fence_proxy_async_shared();     // generic-proxy smem writes -> tensor core
+        mbarrier_arrive(a_ready_bar);
       }
     }
   }
-  tc_fence_before();
+  tcgen05_fence_before();
   __syncthreads();
   if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TC_TMEM_COLS)
-                 : "memory");
+    tcgen05_fence_after();
+    tcgen05_dealloc(tmem_base, TC_TMEM_COLS);
   }
 }
 
@@ -485,7 +380,7 @@ struct TcGemmArgs {
 __global__ void __launch_bounds__(TC_THREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, TcGemmArgs g) {
   extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // keeps the shared address space (LDS/STS)
+  uint8_t* smem = smem_raw + smem_pad1024(smem_raw);
   const int N = g.N;
   const uint32_t a_bytes = TC_BM * 128, w_bytes = (uint32_t)N * 128;
   const uint32_t stage_bytes = a_bytes + w_bytes;
@@ -505,23 +400,21 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < STAGES; ++s) {
-      mbar_init(&full_bar[s], 1);
-      mbar_init(&empty_bar[s], 1);
+      mbarrier_init(&full_bar[s], 1);
+      mbarrier_init(&empty_bar[s], 1);
     }
-    mbar_init(tmem_full_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&map_a)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&map_b)) : "memory");
+    mbarrier_init(tmem_full_bar, 1);
+    fence_mbarrier_init();
+    prefetch_tensormap(&map_a);
+    prefetch_tensormap(&map_b);
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(256u)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tcgen05_alloc(tmem_slot, 256u);
+    tcgen05_relinquish_alloc_permit();
   }
-  tc_fence_before();
+  tcgen05_fence_before();
   __syncthreads();
-  tc_fence_after();
+  tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (num_kb > 0) {
@@ -530,34 +423,35 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         for (int i = 0; i < num_kb; ++i) {
           const int s = i % STAGES;
           const uint32_t ph = (uint32_t)(i / STAGES) & 1u;
-          mbar_wait(&empty_bar[s], ph ^ 1u);
+          mbarrier_wait<TC_SPIN_LOG2>(&empty_bar[s], ph ^ 1u);
           uint8_t* st = smem + (size_t)s * stage_bytes;
-          mbar_arrive_expect_tx(&full_bar[s], stage_bytes);
+          mbarrier_arrive_expect_tx(&full_bar[s], stage_bytes);
           tma_load_2d(st, &map_a, &full_bar[s], (kb0 + i) * TC_BK, m0);
           tma_load_2d(st + a_bytes, &map_b, &full_bar[s], (kb0 + i) * TC_BK, 0);
         }
       }
     } else if (warp == 1) {
       if (lane == 0) {
-        const uint32_t idesc = umma_idesc_tf32(N);
+        const uint32_t idesc = umma_idesc_m128(UMMA_TF32, N);
         for (int i = 0; i < num_kb; ++i) {
           const int s = i % STAGES;
           const uint32_t ph = (uint32_t)(i / STAGES) & 1u;
-          mbar_wait(&full_bar[s], ph);
-          tc_fence_after();
+          mbarrier_wait<TC_SPIN_LOG2>(&full_bar[s], ph);
+          tcgen05_fence_after();
           const uint32_t a_addr = smem_u32(smem + (size_t)s * stage_bytes);
           const uint32_t b_addr = a_addr + a_bytes;
 #pragma unroll
           for (int kk = 0; kk < TC_BK / 8; ++kk)
-            umma_tf32(tmem_base, umma_desc_sw128(a_addr + kk * 32), umma_desc_sw128(b_addr + kk * 32), idesc,
+            tcgen05_mma_tf32(tmem_base, umma_desc_kmajor(a_addr + kk * 32, 1024, UMMA_SWIZZLE_128B),
+                             umma_desc_kmajor(b_addr + kk * 32, 1024, UMMA_SWIZZLE_128B), idesc,
                       (i > 0 || kk > 0) ? 1u : 0u);
-          umma_commit(&empty_bar[s]);
+          tcgen05_commit(&empty_bar[s]);
         }
-        umma_commit(tmem_full_bar);
+        tcgen05_commit(tmem_full_bar);
       }
     } else {
-      mbar_wait(tmem_full_bar, 0);
-      tc_fence_after();
+      mbarrier_wait<TC_SPIN_LOG2>(tmem_full_bar, 0);
+      tcgen05_fence_after();
       const int quarter = warp & 3;
       const int row = m0 + quarter * 32 + lane;
       const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16);
@@ -566,8 +460,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         crow = row < g.msplit ? g.C0 + (size_t)row * g.ldc : g.C1 + (size_t)(row - g.msplit) * g.ldc;
       for (int c = 0; c < N; c += 16) {
         float v[16];
-        tmem_ld16(taddr + c, v);
-        tmem_ld_wait();
+        tcgen05_ld_32x32b_x16(taddr + c, v);
+        tcgen05_wait_ld();
         if (crow != nullptr) {
 #pragma unroll
           for (int j = 0; j < 16; ++j) {
@@ -580,47 +474,12 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       }
     }
   }
-  tc_fence_before();
+  tcgen05_fence_before();
   __syncthreads();
   if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(256u) : "memory");
+    tcgen05_fence_after();
+    tcgen05_dealloc(tmem_base, 256u);
   }
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,
-                                  CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
-                                  CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-    else
-      (void)cudaGetLastError();
-  }
-  return fn;
-}
-
-// 2-D fp32 tensor (rows x cols, row stride ld elements), box = box_rows x 32 cols, 128B swizzle
-bool make_map(EncodeTiledFn enc, CUtensorMap* map, const float* base, int rows, int cols, int ld, int box_rows,
-              int bk = TC_BK) {
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * sizeof(float)};
-  cuuint32_t box[2] = {(cuuint32_t)bk, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, bk == 32 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
-                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS;
 }
 
 }  // namespace
@@ -637,16 +496,16 @@ int glu_gemm_tc(int M, int N, int K, const float* A, int lda, const float* Wl, c
   if (save_l != nullptr && ((lds & 3) || (reinterpret_cast<uintptr_t>(save_l) & 15) ||
                             (reinterpret_cast<uintptr_t>(save_s) & 15)))
     return -1;
-  EncodeTiledFn enc = get_encode_fn();
-  if (enc == nullptr) return -1;
   // CTA pairs with multicast weights unless disabled (STEMGNN_GLU_NO_MULTICAST) or N/2 breaks the 8-row atom
   static const bool no_mc = getenv("STEMGNN_GLU_NO_MULTICAST") != nullptr;
   const int csz = (!no_mc && (N % 16 == 0)) ? 2 : 1;
   const int bk = 32;      // (the 64-byte-row / 5-stage variant of round 1 measured no gain and was removed)
   const int nstage = bk == 32 ? 2 : 5;
+  const CUtensorMapSwizzle sw = bk == 32 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
   CUtensorMap ma, ml, mr;
-  if (!make_map(enc, &ma, A, M, K, lda, TC_BM, bk) || !make_map(enc, &ml, Wl, N, K, K, N / csz, bk) ||
-      !make_map(enc, &mr, Wr, N, K, K, N / csz, bk))
+  if (!make_tensor_map_2d(&ma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, A, M, K, lda * 4ull, TC_BM, bk, sw) ||
+      !make_tensor_map_2d(&ml, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, Wl, N, K, K * 4ull, N / csz, bk, sw) ||
+      !make_tensor_map_2d(&mr, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, Wr, N, K, K * 4ull, N / csz, bk, sw))
     return -1;
   const size_t smem = (size_t)nstage * ((size_t)TC_BM * bk * 4 + 2 * (size_t)N * bk * 4) + 128 +
                       2 * (size_t)N * sizeof(float) + 1024;
@@ -697,10 +556,11 @@ int tc_gemm(int M, int N, int K, float alpha, const float* A, int lda, const flo
     const int rc = tc3_gemm(M, N, K, alpha, A, lda, B, ldb, n_rows_b, C0, C1, msplit, ldc, n_store, atomic, splits, 1, st);
     if (rc >= 0) return rc;
   }
-  EncodeTiledFn enc = get_encode_fn();
-  if (enc == nullptr) return -1;
   CUtensorMap ma, mb;
-  if (!make_map(enc, &ma, A, M, K, lda, TC_BM) || !make_map(enc, &mb, B, n_rows_b, K, ldb, N)) return -1;
+  const CUtensorMapSwizzle sw = CU_TENSOR_MAP_SWIZZLE_128B;
+  if (!make_tensor_map_2d(&ma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, A, M, K, lda * 4ull, TC_BM, TC_BK, sw) ||
+      !make_tensor_map_2d(&mb, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, B, n_rows_b, K, ldb * 4ull, N, TC_BK, sw))
+    return -1;
   const size_t smem = (size_t)3 * (TC_BM * 128 + (size_t)N * 128) + 64 + 1024;
   if (smem > 227 * 1024) return -1;
   static size_t smem_set_dev[64] = {};   // function attributes are per device (ADVICE r1)
@@ -733,14 +593,14 @@ int glu_chain_tc(int M, int N, int K1, const float* G, int ldg, const float* con
   for (int l = 0; l < 3; ++l)
     for (int sd = 0; sd < 2; ++sd)
       if (reinterpret_cast<uintptr_t>(w[l][sd]) & 15) return -1;
-  EncodeTiledFn enc = get_encode_fn();
-  if (enc == nullptr) return -1;
   CUtensorMap mg, mw[3][2];
-  if (!make_map(enc, &mg, G, M, K1, ldg, TC_BM, 32)) return -1;
+  if (!make_tensor_map_2d(&mg, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, G, M, K1, ldg * 4ull, TC_BM, 32, CU_TENSOR_MAP_SWIZZLE_128B))
+    return -1;
   for (int l = 0; l < 3; ++l)
     for (int sd = 0; sd < 2; ++sd) {
       const int K = l == 0 ? K1 : N;
-      if (!make_map(enc, &mw[l][sd], w[l][sd], N, K, K, N, 16)) return -1;
+      if (!make_tensor_map_2d(&mw[l][sd], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, w[l][sd], N, K, K * 4ull, N, 16, CU_TENSOR_MAP_SWIZZLE_64B))
+        return -1;
     }
   const size_t smem = (size_t)8 * TC_BM * 128 + (size_t)3 * 2 * N * 64 + 128 + (size_t)6 * N * sizeof(float) + 1024;
   if (smem > 227 * 1024) return -1;

@@ -25,6 +25,7 @@
 #include "common.cuh"
 #include "gemm.cuh"
 #include "internal.cuh"
+#include "sm100.cuh"
 
 namespace cg = cooperative_groups;
 
@@ -33,51 +34,7 @@ namespace sg {
 
 constexpr int GRU_WARPS = 8;
 constexpr int GRU_THREADS = GRU_WARPS * 32;
-
-__device__ __forceinline__ void cluster_arrive_release() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n" ::: "memory");
-}
-__device__ __forceinline__ void cluster_wait_acquire() {
-  asm volatile("barrier.cluster.wait.acquire.aligned;\n" ::: "memory");
-}
-
-__device__ __forceinline__ uint32_t smem_addr_u32(const void* p) {
-  return static_cast<uint32_t>(__cvta_generic_to_shared(p));
-}
-// shared::cta address -> shared::cluster address of the same variable in CTA `rank`
-__device__ __forceinline__ uint32_t map_to_cta(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-// 16-byte remote store that signals `bytes` on the destination CTA's mbarrier when it lands
-__device__ __forceinline__ void st_async_v4(uint32_t remote_addr, float4 v, uint32_t remote_bar) {
-  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.b32 [%0], {%1, %2, %3, %4}, [%5];"
-               ::"r"(remote_addr), "r"(__float_as_uint(v.x)), "r"(__float_as_uint(v.y)),
-               "r"(__float_as_uint(v.z)), "r"(__float_as_uint(v.w)), "r"(remote_bar)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_init_(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_addr_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx_(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr_u32(bar)), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait_cluster_(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = smem_addr_u32(bar);
-  uint32_t done = 0;
-  for (uint32_t spin = 0; !done; ++spin) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-    if (spin > (1u << 24)) __trap();   // a lost signal must fail loudly, never hang the GPU
-  }
-}
+constexpr int GRU_SPIN_LOG2 = 24;       // mbarrier polls before a lost signal traps
 
 // Warp-wide sum of C values per lane (C a power of two <= 32) by recursive halving: after log2(C)
 // exchange stages every lane owns ONE column sum; lane l ends with the total of value l / (32/C).
@@ -132,10 +89,6 @@ __device__ __forceinline__ void warp_reduce_to_smem(const float* vals, float* ou
   }
 }
 
-// Fast gate nonlinearities (ex2.approx + approximate division: ~2 ulp, abs error < 3e-7 on the gates)
-__device__ __forceinline__ float fast_sigmoid(float x) { return __fdividef(1.0f, 1.0f + __expf(-x)); }
-__device__ __forceinline__ float fast_tanh(float x) { return 2.0f * fast_sigmoid(2.0f * x) - 1.0f; }
-
 // JC: padded h length = 128*JC;  UPW: hidden units per warp;  CS: cluster size;
 // NG x G: a cluster owns NG independent groups of G sequences.  With NG = 2 the groups are software
 // pipelined: while group A's new hidden slices travel through DSMEM, the CTA computes group B.
@@ -184,8 +137,8 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_cluster_kernel(GruArgs a) 
   for (int idx = tid; idx < NG * 5 * G * 32; idx += GRU_THREADS) stage[idx] = 0.f;
   if (tid == 0) {
 #pragma unroll
-    for (int i = 0; i < NG * 2; ++i) mbar_init_(&hbar[i], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int i = 0; i < NG * 2; ++i) mbarrier_init(&hbar[i], 1);
+    fence_mbarrier_init();
   }
   const uint32_t tx_bytes = (uint32_t)(CS * G * UP * sizeof(float));   // bytes a CTA receives per group-step
 
@@ -204,8 +157,8 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_cluster_kernel(GruArgs a) 
       const int rem = idx - dest * (G * UP4);
       const int bb = rem / UP4, i4 = rem - bb * UP4;
       snd_src[it] = bb * 32 + 4 * i4;
-      snd_dst[it] = map_to_cta(smem_addr_u32(hbuf + bb * KP + q * UP + 4 * i4), (uint32_t)dest);
-      snd_bar[it] = map_to_cta(smem_addr_u32(&hbar[0]), (uint32_t)dest);
+      snd_dst[it] = mapa_shared_cluster(smem_u32(hbuf + bb * KP + q * UP + 4 * i4), (uint32_t)dest);
+      snd_bar[it] = mapa_shared_cluster(smem_u32(&hbar[0]), (uint32_t)dest);
     }
   }
 
@@ -258,8 +211,8 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_cluster_kernel(GruArgs a) 
       float* hb_cur = hbuf + ((g * 2 + cur) * G) * KP;
       float* stg = stage + g * 5 * G * 32;
       // arm the barrier of the buffer that will receive h_s, wait until h_{s-1} of this group landed
-      if (tid == 0 && s + 1 < N) mbar_expect_tx_(&hbar[g * 2 + nxt], tx_bytes * (uint32_t)a.xrep);
-      if (s > 0) mbar_wait_cluster_(&hbar[g * 2 + cur], (uint32_t)((s - 1) >> 1) & 1u);
+      if (tid == 0 && s + 1 < N) mbarrier_arrive_expect_tx(&hbar[g * 2 + nxt], tx_bytes * (uint32_t)a.xrep);
+      if (s > 0) mbarrier_wait<GRU_SPIN_LOG2>(&hbar[g * 2 + cur], (uint32_t)((s - 1) >> 1) & 1u);
       float nx_r = 0.f, nx_z = 0.f, nx_n = 0.f;
       if (s + 1 < N) load_gi(s + 1, b0 + g * G + fb, bvalid[g], nx_r, nx_z, nx_n);
 
@@ -331,12 +284,12 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_cluster_kernel(GruArgs a) 
 #pragma unroll
           for (int it = 0; it < SEND_ITEMS; ++it)
             if (snd_src[it] >= 0)
-              st_async_v4(snd_dst[it] + dst_off, *reinterpret_cast<const float4*>(stg + snd_src[it]),
+              st_async_v4(snd_dst[it] + dst_off, *reinterpret_cast<const uint4*>(stg + snd_src[it]),
                           snd_bar[it] + bar_off);
 #pragma unroll
         for (int it = 0; it < SEND_ITEMS; ++it) {
           if (snd_src[it] >= 0) {
-            const float4 v = *reinterpret_cast<const float4*>(stg + snd_src[it]);
+            const uint4 v = *reinterpret_cast<const uint4*>(stg + snd_src[it]);
             st_async_v4(snd_dst[it] + dst_off, v, snd_bar[it] + bar_off);
           }
         }
@@ -492,9 +445,9 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_bwd_cluster_kernel(GruBwdC
   for (int idx = tid; idx < 2 * CS * G * 32; idx += GRU_THREADS) recv[idx] = 0.f;
   for (int idx = tid; idx < 3 * ULOC * G; idx += GRU_THREADS) coef[idx] = make_float2(0.f, 0.f);
   if (tid == 0) {
-    mbar_init_(&rbar[0], 1);
-    mbar_init_(&rbar[1], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbarrier_init(&rbar[0], 1);
+    mbarrier_init(&rbar[1], 1);
+    fence_mbarrier_init();
   }
   const uint32_t tx_bytes = (uint32_t)(CS * G * UP * sizeof(float));
 
@@ -513,8 +466,8 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_bwd_cluster_kernel(GruBwdC
       const int dest = kq / UP4, i4 = kq - dest * UP4;
       if (dest < CS) {
         it_off[it] = bb * KP + 4 * kq;
-        it_dst[it] = map_to_cta(smem_addr_u32(recv + (q * G + bb) * 32 + 4 * i4), (uint32_t)dest);
-        it_bar[it] = map_to_cta(smem_addr_u32(&rbar[0]), (uint32_t)dest);
+        it_dst[it] = mapa_shared_cluster(smem_u32(recv + (q * G + bb) * 32 + 4 * i4), (uint32_t)dest);
+        it_bar[it] = mapa_shared_cluster(smem_u32(&rbar[0]), (uint32_t)dest);
       }
     }
   }
@@ -549,8 +502,8 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_bwd_cluster_kernel(GruBwdC
 
   for (int s = N - 1; s >= 0; --s) {
     const int cur = s & 1, nxt = cur ^ 1;
-    if (tid == 0 && s > 0) mbar_expect_tx_(&rbar[nxt], tx_bytes);
-    if (s < N - 1) mbar_wait_cluster_(&rbar[cur], (uint32_t)((N - 2 - s) >> 1) & 1u);
+    if (tid == 0 && s > 0) mbarrier_arrive_expect_tx(&rbar[nxt], tx_bytes);
+    if (s < N - 1) mbarrier_wait<GRU_SPIN_LOG2>(&rbar[cur], (uint32_t)((N - 2 - s) >> 1) & 1u);
     float nr = 0.f, nz = 0.f, nn = 0.f, nhn = 0.f, nhp = 0.f;
     if (s > 0) load_gates(s - 1, nr, nz, nn, nhn, nhp);
     // (i) gate gradients of the own units
@@ -621,7 +574,9 @@ __global__ void __launch_bounds__(GRU_THREADS, 1) gru_bwd_cluster_kernel(GruBwdC
           const float4 t = *reinterpret_cast<const float4*>(red + (long long)ww * G * KP + it_off[it]);
           v.x += t.x; v.y += t.y; v.z += t.z; v.w += t.w;
         }
-        st_async_v4(it_dst[it] + (uint32_t)nxt * (CS * G * 32 * 4), v, it_bar[it] + (uint32_t)nxt * 8);
+        st_async_v4(it_dst[it] + (uint32_t)nxt * (CS * G * 32 * 4),
+                    make_uint4(__float_as_uint(v.x), __float_as_uint(v.y), __float_as_uint(v.z), __float_as_uint(v.w)),
+                    it_bar[it] + (uint32_t)nxt * 8);
       }
     }
   }

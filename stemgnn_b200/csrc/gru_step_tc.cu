@@ -12,12 +12,11 @@
 //     launch reads as its B operand (kernel boundary = the grid-wide exchange of h).
 // Bound: L2 -> SM streaming of the W_hh images (2 * 3N * N * 2 bytes per step = 50 MB at N = 2048, ~10 us at the measured
 // ~5-6 TB/s L2 rate) — DESIGN.md §8.  The round-1 per-step FFMA path (gru_step_kernel) took ~130 us per step.
-#include <cuda.h>
-#include <cuda_fp16.h>
 #include <stdlib.h>
 
 #include "common.cuh"
 #include "internal.cuh"
+#include "sm100.cuh"
 
 namespace sg {
 namespace {
@@ -30,81 +29,10 @@ constexpr uint32_t ST_A_BYTES = 128 * 128;        // one A tile (128 rows x 64 f
 constexpr uint32_t ST_B_BYTES = 64 * 128;         // B tile (64 rows x 64 fp16)
 constexpr uint32_t ST_STAGE = 2 * ST_A_BYTES + ST_B_BYTES;
 constexpr uint32_t ST_TMEM_COLS = 128;
-constexpr float ST_LO_SCALE = 2048.0f, ST_LO_INV = 1.0f / 2048.0f, ST_LO_INV2 = 1.0f / (2048.0f * 2048.0f);
+constexpr float ST_LO_INV = 1.0f / F16_LO_SCALE, ST_LO_INV2 = 1.0f / (F16_LO_SCALE * F16_LO_SCALE);
+constexpr int ST_SPIN_LOG2 = 26;        // mbarrier polls before a lost arrival traps
 
-__device__ __forceinline__ uint32_t sa(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-__device__ __forceinline__ void mbi(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(sa(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(sa(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbw(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = sa(bar);
-  uint32_t done = 0;
-  for (uint32_t spin = 0; !done; ++spin) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-    if (spin > (1u << 26)) __trap();
-  }
-}
-__device__ __forceinline__ void tma2(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(sa(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(sa(bar)), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void tfb() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tfa() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ uint32_t el1() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}" : "=r"(pred));
-  return pred;
-}
-__device__ __forceinline__ uint64_t dsc128(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr >> 4) & 0x3FFFu);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(1024 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-constexpr uint32_t ST_IDESC = (1u << 4) | ((64u >> 3) << 17) | ((128u >> 4) << 24);     // fp16 x fp16 -> fp32, M128 N64
-__device__ __forceinline__ void mma(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(ST_IDESC), "r"(acc)
-      : "memory");
-}
-__device__ __forceinline__ void cmt(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(sa(bar)) : "memory");
-}
-__device__ __forceinline__ void tld16(uint32_t taddr, float (&v)[16]) {
-  uint32_t r[16];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-#pragma unroll
-  for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void tldw() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ float fsig(float x) { return __fdividef(1.0f, 1.0f + __expf(-x)); }
-__device__ __forceinline__ float ftanh(float x) { return 2.0f * fsig(2.0f * x) - 1.0f; }
-__device__ __forceinline__ void split16(float x, unsigned short& hi, unsigned short& lo) {
-  const __half h = __float2half_rn(x);
-  hi = __half_as_ushort(h);
-  lo = __half_as_ushort(__float2half_rn((x - __half2float(h)) * ST_LO_SCALE));
-}
+constexpr uint32_t ST_IDESC = umma_idesc_m128(UMMA_F16, 64);     // fp16 x fp16 -> fp32, M128 N64
 
 // W_hh (3N, N) fp32 -> image rows [(tile * 2 + arr) * 128 + (gate * 40 + lu)][KP] fp16 (rows 120..127 and pads zero)
 __global__ void __launch_bounds__(256) step_pack_whh_kernel(const float* __restrict__ w_hh, unsigned short* __restrict__ img,
@@ -122,7 +50,7 @@ __global__ void __launch_bounds__(256) step_pack_whh_kernel(const float* __restr
       if (u < N) v = __ldg(w_hh + ((size_t)gate * N + u) * N + k);
     }
     unsigned short hi, lo;
-    split16(v, hi, lo);
+    split_f16_hi_lo_scaled(v, hi, lo);
     img[((size_t)(q * 2 + 0) * 128 + row) * KP + k] = hi;
     img[((size_t)(q * 2 + 1) * 128 + row) * KP + k] = lo;
   }
@@ -140,15 +68,14 @@ struct StepArgs {
 __global__ void __launch_bounds__(ST_THREADS, 1)
 gru_step_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUtensorMap map_h, StepArgs t) {
   extern __shared__ uint8_t smem_raw[];
-  // aligned by pointer arithmetic on the __shared__ array (an integer round trip demotes every access to generic LD/ST)
-  uint8_t* smem = smem_raw + ((1024u - (sa(smem_raw) & 1023u)) & 1023u);
+  uint8_t* smem = smem_raw + smem_pad1024(smem_raw);
   uint8_t* stages = smem;
   float* gh_sm = reinterpret_cast<float*>(stages + ST_NSTG * ST_STAGE);     // [120][32]
   float* wih_sm = gh_sm + 3 * ST_U * ST_SEQ;                                 // [120][W]
   float* bias_sm = wih_sm + 3 * ST_U * t.a.W;                                // [4][40]
   float* x_sm = bias_sm + 4 * ST_U;                                          // [32][W]
   uint8_t* bar_base = reinterpret_cast<uint8_t*>(x_sm + ST_SEQ * t.a.W);
-  bar_base += (8u - (sa(bar_base) & 7u)) & 7u;
+  bar_base += (8u - (smem_u32(bar_base) & 7u)) & 7u;
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(bar_base);
   uint64_t* empty_bar = full_bar + ST_NSTG;
   uint64_t* tfull = empty_bar + ST_NSTG;
@@ -163,16 +90,15 @@ gru_step_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_const
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < ST_NSTG; ++i) {
-      mbi(&full_bar[i], 1);
-      mbi(&empty_bar[i], 1);
+      mbarrier_init(&full_bar[i], 1);
+      mbarrier_init(&empty_bar[i], 1);
     }
-    mbi(tfull, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbarrier_init(tfull, 1);
+    fence_mbarrier_init();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(sa(tmem_slot)), "r"(ST_TMEM_COLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tcgen05_alloc(tmem_slot, ST_TMEM_COLS);
+    tcgen05_relinquish_alloc_permit();
   }
   if (warp >= 2) {      // step-local constants for the gate phase
     const int et = threadIdx.x - 64;
@@ -198,22 +124,22 @@ gru_step_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_const
       x_sm[i] = (b0 + bb) < B ? __ldg(a.xs + ((size_t)s * B + b0 + bb) * W + tt) : 0.f;
     }
   }
-  tfb();
+  tcgen05_fence_before();
   __syncthreads();
-  tfa();
+  tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0) {
-    if (el1()) {        // ===== TMA producer =====
+    if (elect_one_sync()) {        // ===== TMA producer =====
       for (int c = 0; c < t.NCH; ++c) {
         const int st = c % ST_NSTG;
         const uint32_t ph = (uint32_t)(c / ST_NSTG) & 1u;
-        mbw(&empty_bar[st], ph ^ 1u);
+        mbarrier_wait<ST_SPIN_LOG2>(&empty_bar[st], ph ^ 1u);
         uint8_t* dst = stages + (size_t)st * ST_STAGE;
-        mbx(&full_bar[st], ST_STAGE);
-        tma2(dst, &map_w, &full_bar[st], c * 64, (q * 2 + 0) * 128);
-        tma2(dst + ST_A_BYTES, &map_w, &full_bar[st], c * 64, (q * 2 + 1) * 128);
-        tma2(dst + 2 * ST_A_BYTES, &map_h, &full_bar[st], c * 64, (cur * (int)gridDim.y + grp) * 64);
+        mbarrier_arrive_expect_tx(&full_bar[st], ST_STAGE);
+        tma_load_2d(dst, &map_w, &full_bar[st], c * 64, (q * 2 + 0) * 128);
+        tma_load_2d(dst + ST_A_BYTES, &map_w, &full_bar[st], c * 64, (q * 2 + 1) * 128);
+        tma_load_2d(dst + 2 * ST_A_BYTES, &map_h, &full_bar[st], c * 64, (cur * (int)gridDim.y + grp) * 64);
       }
     }
     __syncwarp();
@@ -222,19 +148,20 @@ gru_step_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_const
     for (int c = 0; c < t.NCH; ++c) {
       const int st = c % ST_NSTG;
       const uint32_t ph = (uint32_t)(c / ST_NSTG) & 1u;
-      mbw(&full_bar[st], ph);
-      tfa();
-      if (el1()) {
-        const uint32_t a_hi = sa(stages + (size_t)st * ST_STAGE), a_lo = a_hi + ST_A_BYTES, bt = a_lo + ST_A_BYTES;
+      mbarrier_wait<ST_SPIN_LOG2>(&full_bar[st], ph);
+      tcgen05_fence_after();
+      if (elect_one_sync()) {
+        const uint32_t a_hi = smem_u32(stages + (size_t)st * ST_STAGE), a_lo = a_hi + ST_A_BYTES, bt = a_lo + ST_A_BYTES;
 #pragma unroll
         for (int kk = 0; kk < 4; ++kk) {
-          const uint64_t bd = dsc128(bt + kk * 32);
+          const uint64_t bd = umma_desc_kmajor(bt + kk * 32, 1024, UMMA_SWIZZLE_128B);
           const uint32_t acc = (c > 0 || kk > 0) ? 1u : 0u;
-          mma(tmem_base, dsc128(a_hi + kk * 32), bd, acc);            // W_hi . [h_hi | h_lo]
-          mma(tmem_base + 64, dsc128(a_lo + kk * 32), bd, acc);       // W_lo . [h_hi | h_lo]
+          // W_hi . [h_hi | h_lo], then W_lo . [h_hi | h_lo]
+          tcgen05_mma_f16(tmem_base, umma_desc_kmajor(a_hi + kk * 32, 1024, UMMA_SWIZZLE_128B), bd, ST_IDESC, acc);
+          tcgen05_mma_f16(tmem_base + 64, umma_desc_kmajor(a_lo + kk * 32, 1024, UMMA_SWIZZLE_128B), bd, ST_IDESC, acc);
         }
-        cmt(&empty_bar[st]);
-        if (c + 1 == t.NCH) cmt(tfull);
+        tcgen05_commit(&empty_bar[st]);
+        if (c + 1 == t.NCH) tcgen05_commit(tfull);
       }
       __syncwarp();
     }
@@ -244,24 +171,24 @@ gru_step_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_const
     const int quarter = warp & 3;
     const int row = quarter * 32 + lane;
     const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16);
-    mbw(tfull, 0);
-    tfa();
+    mbarrier_wait<ST_SPIN_LOG2>(tfull, 0);
+    tcgen05_fence_after();
 #pragma unroll
     for (int half = 0; half < 2; ++half) {            // 16 sequences at a time; every lane takes part in the aligned loads
       float d00[16], d01[16], d10[16], d11[16];
-      tld16(taddr + half * 16, d00);                   // W_hi.h_hi
-      tld16(taddr + 32 + half * 16, d01);              // W_hi.h_lo
-      tld16(taddr + 64 + half * 16, d10);              // W_lo.h_hi
-      tld16(taddr + 96 + half * 16, d11);              // W_lo.h_lo
-      tldw();
+      tcgen05_ld_32x32b_x16(taddr + half * 16, d00);                   // W_hi.h_hi
+      tcgen05_ld_32x32b_x16(taddr + 32 + half * 16, d01);              // W_hi.h_lo
+      tcgen05_ld_32x32b_x16(taddr + 64 + half * 16, d10);              // W_lo.h_hi
+      tcgen05_ld_32x32b_x16(taddr + 96 + half * 16, d11);              // W_lo.h_lo
+      tcgen05_wait_ld();
       if (row < 3 * ST_U) {                            // rows 120..127 hold no unit
 #pragma unroll
         for (int j = 0; j < 16; ++j)
           gh_sm[row * ST_SEQ + half * 16 + j] = d00[j] + (d01[j] + d10[j]) * ST_LO_INV + d11[j] * ST_LO_INV2;
       }
     }
-    tfb();
-    asm volatile("bar.sync 1, 128;" ::: "memory");
+    tcgen05_fence_before();
+    bar_sync<1, 128>();
     // gate phase: thread -> sequence b = et % 32, units lu = et / 32 + 4 i
     const int bb = et & 31;
     const int bglob = b0 + bb;
@@ -286,7 +213,7 @@ gru_step_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_const
         const float gh_n = gh_sm[(2 * ST_U + lu) * ST_SEQ + bb] + bias_sm[3 * ST_U + lu];
         const size_t so = (size_t)u * t.Bp + bglob;
         const float hprev = s > 0 ? t.hstate[so] : 0.f;
-        const float r = fsig(gr + gh_r), z = fsig(gz + gh_z), n = ftanh(gn + r * gh_n);
+        const float r = fast_sigmoid(gr + gh_r), z = fast_sigmoid(gz + gh_z), n = fast_tanh(gn + r * gh_n);
         hn = (1.f - z) * n + z * hprev;
         t.hstate[so] = hn;
         t.keyT[so] = fmaf(hn, wk_s, s > 0 ? t.keyT[so] : 0.f);
@@ -301,17 +228,17 @@ gru_step_tc_kernel(const __grid_constant__ CUtensorMap map_w, const __grid_const
       }
       if (u < t.KP) {      // fp16 hi / lo image of h_s: the B operand of the next launch
         unsigned short hi, lo;
-        split16(hn, hi, lo);
+        split_f16_hi_lo_scaled(hn, hi, lo);
         hnext[(size_t)bb * t.KP + u] = hi;
         hnext[(size_t)(32 + bb) * t.KP + u] = lo;
       }
     }
   }
-  tfb();
+  tcgen05_fence_before();
   __syncthreads();
   if (warp == 1) {
-    tfa();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(ST_TMEM_COLS) : "memory");
+    tcgen05_fence_after();
+    tcgen05_dealloc(tmem_base, ST_TMEM_COLS);
   }
 }
 
@@ -327,34 +254,6 @@ __global__ void step_finish_kernel(const float* __restrict__ keyT, const float* 
   }
 }
 
-typedef CUresult (*EncFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                          const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                          CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncFn enc_fn() {
-  static EncFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncFn>(p);
-    else
-      (void)cudaGetLastError();
-  }
-  return fn;
-}
-bool map16(EncFn enc, CUtensorMap* map, const void* base, long long rows, int cols, int box_rows) {
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)cols * 2};
-  cuuint32_t box[2] = {64, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 }  // namespace
 
 // bytes of scratch (inside the `gi` region) the step path needs
@@ -368,8 +267,6 @@ int gru_step_tc_forward(const GruArgs& a, uint8_t* scratch, size_t scratch_bytes
   static const bool off = getenv("STEMGNN_GRU_NO_STEP_TC") != nullptr;
   if (off || scratch == nullptr || a.W > 64) return -1;
   if (gru_step_tc_scratch_bytes(a.B, a.N) > scratch_bytes || (reinterpret_cast<uintptr_t>(scratch) & 255)) return -1;
-  EncFn enc = enc_fn();
-  if (enc == nullptr) return -1;
   const int N = a.N, B = a.B;
   const int NT = ceil_div(N, ST_U), NCH = ceil_div(N, 64), KP = NCH * 64, groups = ceil_div(B, ST_SEQ), Bp = groups * ST_SEQ;
   unsigned short* wimg = reinterpret_cast<unsigned short*>(scratch);
@@ -378,7 +275,10 @@ int gru_step_tc_forward(const GruArgs& a, uint8_t* scratch, size_t scratch_bytes
   float* keyT = hstate + (size_t)KP * Bp;
   float* queryT = keyT + (size_t)KP * Bp;
   CUtensorMap mw, mh;
-  if (!map16(enc, &mw, wimg, (long long)NT * 2 * 128, KP, 128) || !map16(enc, &mh, himg, (long long)2 * groups * 64, KP, 64))
+  if (!make_tensor_map_2d(&mw, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, wimg, (uint64_t)NT * 2 * 128, KP, KP * 2ull, 128, 64,
+                          CU_TENSOR_MAP_SWIZZLE_128B) ||
+      !make_tensor_map_2d(&mh, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, himg, (uint64_t)2 * groups * 64, KP, KP * 2ull, 64, 64,
+                          CU_TENSOR_MAP_SWIZZLE_128B))
     return -1;
   const size_t smem = (size_t)ST_NSTG * ST_STAGE + ((size_t)3 * ST_U * ST_SEQ + (size_t)3 * ST_U * a.W + 4 * ST_U +
                                                     (size_t)ST_SEQ * a.W + 2) * sizeof(float) +

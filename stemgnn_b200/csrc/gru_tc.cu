@@ -22,11 +22,11 @@
 // Envelope: N <= 16*40 with (U, CS) such that the tiles fit 227 KB (N <= 448), W <= 64, G <= 8; everything else
 // takes the FFMA2 cluster kernel / per-step path of gru.cu.
 #include <cooperative_groups.h>
-#include <cuda_fp16.h>
 #include <stdlib.h>
 
 #include "common.cuh"
 #include "internal.cuh"
+#include "sm100.cuh"
 
 namespace cg = cooperative_groups;
 
@@ -39,116 +39,12 @@ constexpr int GT_THREADS = (GT_ROUNDS + 4) * 32;   // warps 0..2: MMA issue (war
 constexpr int GT_EPI = 128;
 constexpr int GT_GMAX = 8;             // sequences per cluster (rows 0..7 of the B tile = h_hi, 8..15 = h_lo)
 constexpr uint32_t GT_TMEM_COLS = 512;    // D (32 columns) + the resident W_hh hi/lo operand
-constexpr float GT_LO_SCALE = 2048.0f;             // 2^11
-constexpr float GT_LO_INV = 1.0f / 2048.0f;
-constexpr float GT_LO_INV2 = 1.0f / (2048.0f * 2048.0f);
+constexpr float GT_LO_INV = 1.0f / F16_LO_SCALE;
+constexpr float GT_LO_INV2 = 1.0f / (F16_LO_SCALE * F16_LO_SCALE);
+constexpr int GT_SPIN_LOG2 = 24;       // mbarrier polls before a lost signal traps
 
-__device__ __forceinline__ uint32_t s_u32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-__device__ __forceinline__ uint32_t map_cta(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void st_async_16(uint32_t remote_addr, uint4 v, uint32_t remote_bar) {
-  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.b32 [%0], {%1, %2, %3, %4}, [%5];"
-               ::"r"(remote_addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w), "r"(remote_bar)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(s_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(s_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(s_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = s_u32(bar);
-  uint32_t done = 0;
-  for (uint32_t spin = 0; !done; ++spin) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-    if (spin > (1u << 24)) __trap();   // a lost signal must fail loudly, never hang the GPU
-  }
-}
-// wait on a barrier that is completed by st.async stores of OTHER CTAs of the cluster: acquire at cluster scope
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = s_u32(bar);
-  uint32_t done = 0;
-  for (uint32_t spin = 0; !done; ++spin) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-    if (spin > (1u << 24)) __trap();
-  }
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(s_u32(dst)), "l"(reinterpret_cast<uint64_t>(src)), "r"(bytes), "r"(s_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_proxy() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-// K-major, 128B-swizzled operand tile: rows of 128 bytes (64 fp16 along K), 8-row groups 1024 bytes apart
-__device__ __forceinline__ uint64_t desc_sw128(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr >> 4) & 0x3FFFu);        // start address            bits [0,14)
-  d |= (uint64_t)1 << 16;                             // leading byte offset (unused for swizzled K-major)
-  d |= (uint64_t)(1024 >> 4) << 32;                   // stride byte offset = 1024 bits [32,46)
-  d |= (uint64_t)1 << 46;                             // descriptor version (sm_100)
-  d |= (uint64_t)2 << 61;                             // layout type SWIZZLE_128B
-  return d;
-}
-// kind::f16 instruction descriptor: fp16 A and B (format 0), fp32 accumulate, both K-major, M=128, N=16
-constexpr uint32_t GT_IDESC = (1u << 4) | ((16u >> 3) << 17) | ((128u >> 4) << 24);
-__device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(GT_IDESC), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(s_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-      "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]),
-        "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]),
-        "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-#pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-__device__ __forceinline__ float fast_sigmoid(float x) { return __fdividef(1.0f, 1.0f + __expf(-x)); }
-__device__ __forceinline__ float fast_tanh(float x) { return 2.0f * fast_sigmoid(2.0f * x) - 1.0f; }
-
-// x = hi + lo / 2^11 with hi, lo in fp16 (lo pre-scaled by 2^11 so that it stays in the normal range)
-__device__ __forceinline__ void split_f16(float x, __half& hi, __half& lo) {
-  hi = __float2half_rn(x);
-  lo = __float2half_rn((x - __half2float(hi)) * GT_LO_SCALE);
-}
+// kind::f16 instruction descriptor: fp16 A and B, fp32 accumulate, both K-major, M=128, N=16
+constexpr uint32_t GT_IDESC = umma_idesc_m128(UMMA_F16, 16);
 
 // byte offset of element (row, k) inside a K-major SWIZZLE_128B fp16 operand whose 64-column chunks are
 // `chunk_bytes` apart (16-byte granule index XOR row%8; the tile base is 1024-byte aligned)
@@ -189,11 +85,11 @@ __global__ void __launch_bounds__(128) gru_pack_whh_kernel(const float* __restri
   uint32_t hi[4], lo[4];
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
-    __half h0, l0, h1, l1;
-    split_f16(v[2 * i], h0, l0);
-    split_f16(v[2 * i + 1], h1, l1);
-    hi[i] = (uint32_t)__half_as_ushort(h0) | ((uint32_t)__half_as_ushort(h1) << 16);
-    lo[i] = (uint32_t)__half_as_ushort(l0) | ((uint32_t)__half_as_ushort(l1) << 16);
+    unsigned short h0, l0, h1, l1;
+    split_f16_hi_lo_scaled(v[2 * i], h0, l0);
+    split_f16_hi_lo_scaled(v[2 * i + 1], h1, l1);
+    hi[i] = (uint32_t)h0 | ((uint32_t)h1 << 16);
+    lo[i] = (uint32_t)l0 | ((uint32_t)l1 << 16);
   }
   uint4* base = img + (size_t)q * (a_img_bytes(g) / 16);
   base[(size_t)kg * 128 + row] = make_uint4(hi[0], hi[1], hi[2], hi[3]);
@@ -214,32 +110,11 @@ struct GruTcArgs {
 // elect.sync / tcgen05.ld.sync.aligned breaks those warp-collective instructions (seen as wrong results in early debug builds)
 #define GT_STAMP(slot) do { if (dbg_on) { if (lane == 0) ta.dbg[(s - dbg_s0) * 16 + (slot)] = clock64(); __syncwarp(); } } while (0)
 
-__device__ __forceinline__ void umma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(GT_IDESC), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ uint32_t elect_one() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}" : "=r"(pred));
-  return pred;
-}
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, uint4 a, uint4 b) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
-               ::"r"(taddr), "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w), "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w)
-               : "memory");
-}
-
 // PP = (unit, sequence) pairs per epilogue thread
 template <int PP>
 __global__ void __launch_bounds__(GT_THREADS, 1) gru_tc_cluster_kernel(GruTcArgs ta) {
   extern __shared__ uint8_t smem_raw[];
-  // aligned by pointer arithmetic on the __shared__ array: an integer round trip demotes EVERY shared-memory access of the
-  // step loop to generic LD/ST (612 LD.E + 360 LD.E.128 in the SASS of the previous build)
-  uint8_t* smem = smem_raw + ((1024u - (s_u32(smem_raw) & 1023u)) & 1023u);
+  uint8_t* smem = smem_raw + smem_pad1024(smem_raw);
   const GruArgs& a = ta.a;
   const GruTcGeom g = ta.g;
   const int U = g.U, CS = g.CS, G = ta.G;
@@ -250,16 +125,16 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gru_tc_cluster_kernel(GruTcArgs
   float* gh_sm = reinterpret_cast<float*>(B_sm + 2 * b_buf);          // [128][8]
   float* wih_sm = gh_sm + 128 * GT_GMAX;                  // [3U][W]
   float* bias_sm = wih_sm + 3 * U * W;                    // [3U] b_ih (+ b_hh for r,z) and [U] b_hn
-  __half* stage_sm = reinterpret_cast<__half*>(bias_sm + 4 * U);      // [2][8][U] (16-byte aligned: U % 8 == 0)
+  unsigned short* stage_sm = reinterpret_cast<unsigned short*>(bias_sm + 4 * U);      // [2][8][U] (16-byte aligned: U % 8 == 0)
   uint8_t* hbar_base = reinterpret_cast<uint8_t*>(stage_sm + 2 * GT_GMAX * U);
-  hbar_base += (8u - (s_u32(hbar_base) & 7u)) & 7u;
+  hbar_base += (8u - (smem_u32(hbar_base) & 7u)) & 7u;
   uint64_t* hbar = reinterpret_cast<uint64_t*>(hbar_base);
   uint64_t* tfull = hbar + 2 * 16;                        // hbar[buf][source]
   uint64_t* xbar = tfull + GT_ROUNDS;                     // tfull[r]: accumulator set r complete
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(xbar + 1);
   uint32_t* rdy_sm = tmem_slot + 2;                       // [16] rdy[r]: K steps of round r, rdy[8 + r]: last arrival index of round r
   uint8_t* xs_base = reinterpret_cast<uint8_t*>(rdy_sm + 16);
-  xs_base += (16u - (s_u32(xs_base) & 15u)) & 15u;
+  xs_base += (16u - (smem_u32(xs_base) & 15u)) & 15u;
   float* xs_sm = reinterpret_cast<float*>(xs_base);       // [N][G][W]
 
   cg::cluster_group cluster = cg::this_cluster();
@@ -272,16 +147,14 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gru_tc_cluster_kernel(GruTcArgs
 
   // ---- one-time setup ------------------------------------------------------------------------------------
   if (tid == 0) {
-    for (int i = 0; i < 2 * 16; ++i) mbar_init(&hbar[i], 1);
-    for (int r = 0; r < GT_ROUNDS; ++r) mbar_init(&tfull[r], 1);   // tfull[0] is re-initialised below with the round count
-    mbar_init(xbar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int i = 0; i < 2 * 16; ++i) mbarrier_init(&hbar[i], 1);
+    for (int r = 0; r < GT_ROUNDS; ++r) mbarrier_init(&tfull[r], 1);   // tfull[0] is re-initialised below with the round count
+    mbarrier_init(xbar, 1);
+    fence_mbarrier_init();
   }
   if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(tmem_slot)),
-                 "r"(GT_TMEM_COLS)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tcgen05_alloc(tmem_slot, GT_TMEM_COLS);
+    tcgen05_relinquish_alloc_permit();
   }
   // B tiles (both buffers) start as zeros: h_{-1} = 0, padding columns / unused sequence rows stay zero forever
   for (int i = tid; i < (int)(2 * b_buf / 16); i += GT_THREADS)
@@ -312,10 +185,10 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gru_tc_cluster_kernel(GruTcArgs
       dst[(size_t)ss * pitch + v] = __ldg(src + ((size_t)ss * B + b0) * (W / 4) + v);
     }
   }
-  fence_async_proxy();                 // generic-proxy zero fill -> visible to the tensor core's async proxy
-  tc_fence_before();
+  fence_proxy_async_shared();                 // generic-proxy zero fill -> visible to the tensor core's async proxy
+  tcgen05_fence_before();
   __syncthreads();
-  tc_fence_after();
+  tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   const uint32_t a_cols = (uint32_t)g.NKS * 8u;            // TMEM columns per W_hh array (2 fp16 per column)
 
@@ -343,9 +216,9 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gru_tc_cluster_kernel(GruTcArgs
       if (lane == 0) {                 // ONE accumulator barrier: every non-empty round commits to it once per step
         rdy_sm[12] = (uint32_t)__popc(nz);
         if (nz != 0u) {
-          asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(s_u32(&tfull[0])) : "memory");
-          mbar_init(&tfull[0], (uint32_t)__popc(nz));
-          asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+          mbarrier_inval(&tfull[0]);
+          mbarrier_init(&tfull[0], (uint32_t)__popc(nz));
+          fence_mbarrier_init();
         }
       }
     }
@@ -361,13 +234,13 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gru_tc_cluster_kernel(GruTcArgs
     for (int i = 0; i < nst; ++i) {
       const uint4 v0 = __ldg(src + (size_t)(2 * i) * 128);
       const uint4 v1 = __ldg(src + (size_t)(2 * i + 1) * 128);
-      tmem_st8(tA + (uint32_t)i * 8u, v0, v1);
+      tcgen05_st_32x32b_x8(tA + (uint32_t)i * 8u, v0, v1);
     }
-    asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+    tcgen05_wait_st();
   }
-  tc_fence_before();
+  tcgen05_fence_before();
   cluster.sync();                      // every CTA's tiles and barriers exist before any remote store
-  tc_fence_after();
+  tcgen05_fence_after();
 
   const uint32_t src_bytes = (uint32_t)(2 * G * U * 2);    // bytes a CTA receives per step from ONE source CTA
 
@@ -398,25 +271,26 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gru_tc_cluster_kernel(GruTcArgs
         if (lane <= last) {
           // plain (cta-scope) acquire: the cluster-scope form makes ptxas add CCTL.IVALL (an L1 invalidate, 8 % of the
           // kernel's stall samples in profiles/r02_ncu_gru_tc_stalls.txt) although the payload lives in shared memory
-          mbar_wait(&hbar[cur * 16 + my_p], par);                      // slices of h_{s-1} landed in B[cur]
-          fence_async_proxy();         // every observer orders the remote generic-proxy stores before async-proxy reads
+          mbarrier_wait<GT_SPIN_LOG2>(&hbar[cur * 16 + my_p], par);                      // slices of h_{s-1} landed in B[cur]
+          fence_proxy_async_shared();         // every observer orders the remote generic-proxy stores before async-proxy reads
         }
         __syncwarp();
         GT_STAMP(1);
-        if (elect_one()) {
-          fence_async_proxy();
-          tc_fence_after();
-          const uint32_t b_addr = s_u32(B_sm) + (uint32_t)cur * b_buf;
+        if (elect_one_sync()) {
+          fence_proxy_async_shared();
+          tcgen05_fence_after();
+          const uint32_t b_addr = smem_u32(B_sm) + (uint32_t)cur * b_buf;
           uint32_t todo = todo0, acc = 0u;
           while (todo) {
             const int j = __ffs((int)todo) - 1;
             todo &= todo - 1u;
-            const uint64_t bd = desc_sw128(b_addr + (uint32_t)(j >> 2) * B_CHUNK_BYTES + (uint32_t)(j & 3) * 32u);
-            umma_f16_ts(d0, a_hi + (uint32_t)j * 8u, bd, acc);             // W_hi . [h_hi | h_lo]
-            umma_f16_ts(d0 + 16u, a_lo + (uint32_t)j * 8u, bd, acc);       // W_lo . [h_hi | h_lo]
+            const uint64_t bd = umma_desc_kmajor(b_addr + (uint32_t)(j >> 2) * B_CHUNK_BYTES + (uint32_t)(j & 3) * 32u, 1024,
+                                                 UMMA_SWIZZLE_128B);
+            tcgen05_mma_f16_tmem_a(d0, a_hi + (uint32_t)j * 8u, bd, GT_IDESC, acc);           // W_hi . [h_hi | h_lo]
+            tcgen05_mma_f16_tmem_a(d0 + 16u, a_lo + (uint32_t)j * 8u, bd, GT_IDESC, acc);     // W_lo . [h_hi | h_lo]
             acc = 1u;
           }
-          umma_commit(&tfull[0]);
+          tcgen05_commit(&tfull[0]);
         }
         __syncwarp();
         GT_STAMP(3);
@@ -499,8 +373,8 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gru_tc_cluster_kernel(GruTcArgs
           const int dest = (q + slot) % CS;
           snd_src[i][k] = (uint32_t)(((arr * GT_GMAX + bb) * U + lu0) * 2);                 // bytes into stage_sm
           const uint32_t off = sw128_off(arr * 8 + bb, u0 + lu0, B_CHUNK_BYTES);
-          snd_dst[i][k] = map_cta(s_u32(B_sm) + off, (uint32_t)dest);
-          snd_bar[i][k] = map_cta(s_u32(&hbar[q]), (uint32_t)dest);    // the destination's barrier for source q
+          snd_dst[i][k] = mapa_shared_cluster(smem_u32(B_sm) + off, (uint32_t)dest);
+          snd_bar[i][k] = mapa_shared_cluster(smem_u32(&hbar[q]), (uint32_t)dest);    // the destination's barrier for source q
         }
       }
     }
@@ -511,7 +385,7 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gru_tc_cluster_kernel(GruTcArgs
       const int nxt = (s & 1) ^ 1;
       const bool dbg_on = ta.dbg != nullptr && ta.dbg_mode != 3 && blockIdx.x == 0 && warp == GT_ROUNDS && s >= dbg_s0 && s < dbg_s0 + 4;
       GT_STAMP(4);
-      if (et < CS && s + 1 < N) mbar_expect_tx(&hbar[nxt * 16 + et], src_bytes);   // arm the tile that will receive h_s
+      if (et < CS && s + 1 < N) mbarrier_arrive_expect_tx(&hbar[nxt * 16 + et], src_bytes);   // arm the tile that will receive h_s
       // input projection of the NEXT step while this step's MMAs run
       float nx_r[PP] = {}, nx_z[PP] = {}, nx_n[PP] = {}, nx_wk = 0.f, nx_wq = 0.f;
       if (s + 1 < N) {
@@ -527,15 +401,15 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gru_tc_cluster_kernel(GruTcArgs
         float o[8];
 #pragma unroll
         for (int b = 0; b < 8; ++b) o[b] = 0.f;
-        mbar_wait(&tfull[0], (uint32_t)(s - 1) & 1u);      // every round's MMAs of this step are complete
-        tc_fence_after();
+        mbarrier_wait<GT_SPIN_LOG2>(&tfull[0], (uint32_t)(s - 1) & 1u);      // every round's MMAs of this step are complete
+        tcgen05_fence_after();
         GT_STAMP(6);
         // all accumulator sets are loaded back to back and waited for once: three dependent load -> wait round trips
         // measured ~430 cycles (profiles/r02_gru_phase_stamps.txt)
         float d[GT_ROUNDS][32];
 #pragma unroll
-        for (int r = 0; r < GT_ROUNDS; ++r) tmem_ld32(taddr + 32u * (uint32_t)r, d[r]);
-        tmem_ld_wait();
+        for (int r = 0; r < GT_ROUNDS; ++r) tcgen05_ld_32x32b_x32(taddr + 32u * (uint32_t)r, d[r]);
+        tcgen05_wait_ld();
 #pragma unroll
         for (int r = 0; r < GT_ROUNDS; ++r) {
           if (rdy_sm[r] != 0u) {             // a round without K steps never wrote its set
@@ -548,8 +422,8 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gru_tc_cluster_kernel(GruTcArgs
         float4* gp = reinterpret_cast<float4*>(gh_sm + row * GT_GMAX);
         gp[0] = make_float4(o[0], o[1], o[2], o[3]);
         gp[1] = make_float4(o[4], o[5], o[6], o[7]);
-        tc_fence_before();             // the next step's MMAs (ordered after this thread's sends) overwrite D
-        asm volatile("bar.sync 1, 128;" ::: "memory");
+        tcgen05_fence_before();             // the next step's MMAs (ordered after this thread's sends) overwrite D
+        bar_sync<1, 128>();
         GT_STAMP(8);
       }
 #pragma unroll
@@ -580,8 +454,8 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gru_tc_cluster_kernel(GruTcArgs
             }
             hprev[i] = hn;
           }
-          __half hi, lo;
-          split_f16(hn, hi, lo);
+          unsigned short hi, lo;
+          split_f16_hi_lo_scaled(hn, hi, lo);
           stage_sm[(0 * GT_GMAX + bb) * U + lu] = hi;
           stage_sm[(1 * GT_GMAX + bb) * U + lu] = lo;
         }
@@ -599,7 +473,7 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gru_tc_cluster_kernel(GruTcArgs
           for (int i = 0; i < PP; ++i) {
             if (snd_src[i][k] != 0xFFFFFFFFu) {
               const uint4 v = *reinterpret_cast<const uint4*>(reinterpret_cast<const uint8_t*>(stage_sm) + snd_src[i][k]);
-              st_async_16(snd_dst[i][k] + dst_off, v, snd_bar[i][k] + bar_off);
+              st_async_v4(snd_dst[i][k] + dst_off, v, snd_bar[i][k] + bar_off);
             }
           }
         }
@@ -615,12 +489,11 @@ __global__ void __launch_bounds__(GT_THREADS, 1) gru_tc_cluster_kernel(GruTcArgs
       }
     }
   }
-  tc_fence_before();
+  tcgen05_fence_before();
   cluster.sync();      // no CTA may exit while peers could still address its shared memory
   if (warp == 0) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(GT_TMEM_COLS)
-                 : "memory");
+    tcgen05_fence_after();
+    tcgen05_dealloc(tmem_base, GT_TMEM_COLS);
   }
 }
 

@@ -1,8 +1,16 @@
 // Internal (non-ABI) declarations shared by the stemgnn_b200 translation units.
 #pragma once
+#include <cuda.h>
+
 #include "common.cuh"
 
 namespace sg {
+
+// ---- TMA tensor maps (tensor_map.cu) ------------------------------------------------------------------------------------
+// 2-D tiled map of a row-major `rows` x `cols` tensor with row pitch `pitch_bytes` (anything outside reads as zero), box =
+// box_rows x box_cols elements.  false when the driver has no encoder or rejects the map (callers then return -1).
+bool make_tensor_map_2d(CUtensorMap* map, CUtensorMapDataType dtype, const void* base, uint64_t rows, uint64_t cols,
+                        uint64_t pitch_bytes, uint32_t box_rows, uint32_t box_cols, CUtensorMapSwizzle swizzle);
 
 // ---- GRU (gru.cu) --------------------------------------------------------------------------------
 struct GruArgs {

@@ -28,13 +28,11 @@
 //                 TMEM lane quarter split the columns).  ncu (profiles/r02_ncu_spec_*): these kernels are bound by
 //                 shared-memory bandwidth (TMA fill + split traffic + 3x operand reads) and by the epilogue's latency
 //                 chains, not by the tensor pipe — hence 8 worker warps and the stacked B operand.
-#include <cuda.h>
-#include <cuda_bf16.h>
-#include <cuda_fp16.h>
 #include <stdlib.h>
 
 #include "common.cuh"
 #include "internal.cuh"
+#include "sm100.cuh"
 
 namespace sg {
 namespace {
@@ -44,82 +42,9 @@ constexpr int S_BK = 32;                 // fp32 elements per K block = one 128-
 constexpr int S_THREADS = 320;          // warp 0 TMA, warp 1 MMA issue, warps 2..9 operand split + epilogue
 constexpr int S_WORKERS = 256;
 constexpr uint32_t S_A_BYTES = S_BM * 128;
+constexpr int S_SPIN_LOG2 = 26;         // mbarrier polls before a lost arrival traps
 
 enum { EPI_STORE = 0, EPI_GFT = 1, EPI_HEAD = 2 };
-
-__device__ __forceinline__ uint32_t s32(const void* p) { return static_cast<uint32_t>(__cvta_generic_to_shared(p)); }
-__device__ __forceinline__ void mb_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(s32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mb_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(s32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mb_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(s32(bar)) : "memory");
-}
-__device__ __forceinline__ void mb_wait(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = s32(bar);
-  uint32_t done = 0;
-  for (uint32_t spin = 0; !done; ++spin) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-    if (spin > (1u << 26)) __trap();   // a lost arrival must fail, not hang the GPU
-  }
-}
-__device__ __forceinline__ void tma_2d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(s32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(s32(bar)), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void tcf_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tcf_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ uint32_t elect1() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}" : "=r"(pred));
-  return pred;
-}
-// K-major, 128B-swizzled operand tile: rows of 128 bytes, 8-row groups 1024 bytes apart
-__device__ __forceinline__ uint64_t desc_sw128(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr >> 4) & 0x3FFFu);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(1024 >> 4) << 32;
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
-  return d;
-}
-// kind::tf32, fp32 accumulate, A and B K-major, M = 128
-__device__ __forceinline__ uint32_t idesc_tf32(int n) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(S_BM >> 4) << 24);
-}
-__device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(acc)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(s32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
-  uint32_t r[16];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-        "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-#pragma unroll
-  for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 struct Tc3Args {
   int M, K;            // rows of A that exist, reduction length
@@ -139,18 +64,6 @@ struct Tc3Args {
   const float* x_bnw; float* forecast; float* bc_bnw; float* bc_bwn; float* bc_pad; int ld_pad; float* save_fs; int T;
 };
 
-__device__ __forceinline__ void to_h16(float x, int bf16, unsigned short& hi, unsigned short& lo) {
-  if (bf16) {
-    hi = __bfloat16_as_ushort(__float2bfloat16_rn(x));
-    lo = 0;
-  } else {
-    const float xs = fminf(fmaxf(x, -65504.f), 65504.f);
-    const __half h = __float2half_rn(xs);
-    hi = __half_as_ushort(h);
-    lo = __half_as_ushort(__float2half_rn(xs - __half2float(h)));
-  }
-}
-__device__ __forceinline__ float fast_sigmoid(float x) { return __fdividef(1.0f, 1.0f + __expf(-x)); }
 // lo = x - (x & 0xffffe000).  The `hi` tile is NOT rewritten: kind::tf32 truncates its operands to the top 19 bits (measured:
 // the error of a single pass on seeded inputs equals the truncation model to 3 digits on every tested shape — 6.42e-4 /
 // 9.35e-4 / 7.19e-4 / 7.92e-4 — where round-to-nearest would give 4.18e-4 / 3.83e-4 / 2.76e-4 / 3.78e-4; profiles/README.md),
@@ -171,9 +84,7 @@ template <int EPI>
 __global__ void __launch_bounds__(S_THREADS, 1)
 tc3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, Tc3Args g) {
   extern __shared__ uint8_t smem_raw[];
-  // 1024-byte alignment for the 128B swizzle, by pointer arithmetic on the __shared__ array (an integer round trip would
-  // demote every access below to generic LD/ST)
-  uint8_t* smem = smem_raw + ((1024u - (s32(smem_raw) & 1023u)) & 1023u);
+  uint8_t* smem = smem_raw + smem_pad1024(smem_raw);
   const int NT = g.NT, S = g.nstage;
   const uint32_t b_bytes = (uint32_t)NT * 128;
   const bool split = g.split != 0;
@@ -200,74 +111,77 @@ tc3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CU
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < S; ++s) {
-      mb_init(&full_bar[s], 1);
-      mb_init(&empty_bar[s], 1);
-      mb_init(&conv_bar[s], S_WORKERS);
+      mbarrier_init(&full_bar[s], 1);
+      mbarrier_init(&empty_bar[s], 1);
+      mbarrier_init(&conv_bar[s], S_WORKERS);
     }
-    mb_init(tmem_full_bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&map_a)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&map_b)) : "memory");
+    mbarrier_init(tmem_full_bar, 1);
+    fence_mbarrier_init();
+    prefetch_tensormap(&map_a);
+    prefetch_tensormap(&map_b);
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(tmem_slot)), "r"(g.tmem_cols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    tcgen05_alloc(tmem_slot, g.tmem_cols);
+    tcgen05_relinquish_alloc_permit();
   }
-  tcf_before();
+  tcgen05_fence_before();
   __syncthreads();
-  tcf_after();
+  tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0) {
     // ===== TMA producer =====
-    if (num_kb > 0 && elect1()) {
+    if (num_kb > 0 && elect_one_sync()) {
       for (int i = 0; i < num_kb; ++i) {
         const int s = i % S;
         const uint32_t ph = (uint32_t)(i / S) & 1u;
-        mb_wait(&empty_bar[s], ph ^ 1u);
+        mbarrier_wait<S_SPIN_LOG2>(&empty_bar[s], ph ^ 1u);
         uint8_t* st = smem + (size_t)s * stage_bytes;
-        mb_expect_tx(&full_bar[s], S_A_BYTES + b_bytes);
-        tma_2d(st, &map_a, &full_bar[s], (kb0 + i) * S_BK, m0);
-        tma_2d(st + b_hi_off, &map_b, &full_bar[s], (kb0 + i) * S_BK, n0);
+        mbarrier_arrive_expect_tx(&full_bar[s], S_A_BYTES + b_bytes);
+        tma_load_2d(st, &map_a, &full_bar[s], (kb0 + i) * S_BK, m0);
+        tma_load_2d(st + b_hi_off, &map_b, &full_bar[s], (kb0 + i) * S_BK, n0);
       }
     }
     __syncwarp();
   } else if (warp == 1) {
     // ===== MMA issuer: converged warp, one elected lane =====
     if (num_kb > 0) {
-      const uint32_t idesc = idesc_tf32(NT);
-      const uint32_t idesc2 = idesc_tf32(2 * NT);          // stacked [B_hi; B_lo]
+      const uint32_t idesc = umma_idesc_m128(UMMA_TF32, NT);
+      const uint32_t idesc2 = umma_idesc_m128(UMMA_TF32, 2 * NT);          // stacked [B_hi; B_lo]
       const uint32_t lo_col = g.lo_col;
       const bool stacked = g.stacked != 0;
       for (int i = 0; i < num_kb; ++i) {
         const int s = i % S;
         const uint32_t ph = (uint32_t)(i / S) & 1u;
-        mb_wait(split ? &conv_bar[s] : &full_bar[s], ph);
-        tcf_after();
-        if (elect1()) {
-          const uint32_t a_hi = s32(smem + (size_t)s * stage_bytes);
+        mbarrier_wait<S_SPIN_LOG2>(split ? &conv_bar[s] : &full_bar[s], ph);
+        tcgen05_fence_after();
+        if (elect_one_sync()) {
+          const uint32_t a_hi = smem_u32(smem + (size_t)s * stage_bytes);
           const uint32_t a_lo = a_hi + a_lo_off, b_hi = a_hi + b_hi_off, b_lo = a_hi + b_lo_off;
 #pragma unroll
           for (int kk = 0; kk < S_BK / 8; ++kk) {      // 8 tf32 = 32 bytes along K per instruction
             const uint32_t acc = (i > 0 || kk > 0) ? 1u : 0u;
-            const uint64_t da = desc_sw128(a_hi + kk * 32), db = desc_sw128(b_hi + kk * 32);
+            const uint64_t da = umma_desc_kmajor(a_hi + kk * 32, 1024, UMMA_SWIZZLE_128B);
+            const uint64_t db = umma_desc_kmajor(b_hi + kk * 32, 1024, UMMA_SWIZZLE_128B);
             if (!split) {
-              umma_tf32(tmem_base, da, db, idesc, acc);
+              tcgen05_mma_tf32(tmem_base, da, db, idesc, acc);
             } else if (stacked) {   // hi.hi -> [0,NT), hi.lo -> [NT,2NT) in one instruction; then lo.hi onto [NT,2NT)
-              umma_tf32(tmem_base, da, db, idesc2, acc);
-              umma_tf32(tmem_base + lo_col, desc_sw128(a_lo + kk * 32), db, idesc, 1u);
+              tcgen05_mma_tf32(tmem_base, da, db, idesc2, acc);
+              tcgen05_mma_tf32(tmem_base + lo_col, umma_desc_kmajor(a_lo + kk * 32, 1024, UMMA_SWIZZLE_128B), db, idesc,
+                               1u);
             } else {                // cross terms in their own accumulator (file header)
-              umma_tf32(tmem_base, da, db, idesc, acc);
-              umma_tf32(tmem_base + lo_col, desc_sw128(a_lo + kk * 32), db, idesc, acc);
-              umma_tf32(tmem_base + lo_col, da, desc_sw128(b_lo + kk * 32), idesc, 1u);
+              tcgen05_mma_tf32(tmem_base, da, db, idesc, acc);
+              tcgen05_mma_tf32(tmem_base + lo_col, umma_desc_kmajor(a_lo + kk * 32, 1024, UMMA_SWIZZLE_128B), db, idesc,
+                               acc);
+              tcgen05_mma_tf32(tmem_base + lo_col, da, umma_desc_kmajor(b_lo + kk * 32, 1024, UMMA_SWIZZLE_128B), idesc,
+                               1u);
             }
           }
-          umma_commit(&empty_bar[s]);
+          tcgen05_commit(&empty_bar[s]);
         }
         __syncwarp();
       }
-      if (elect1()) umma_commit(tmem_full_bar);
+      if (elect_one_sync()) tcgen05_commit(tmem_full_bar);
       __syncwarp();
     }
   } else {
@@ -296,7 +210,7 @@ tc3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CU
           s_bsc[i] = __ldg(g.bsc + i);
         }
       }
-      asm volatile("bar.sync 1, 256;" ::: "memory");
+      bar_sync<1, 256>();
     }
     if (num_kb > 0) {
       if (split) {
@@ -305,7 +219,7 @@ tc3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CU
         for (int i = 0; i < num_kb; ++i) {
           const int s = i % S;
           const uint32_t ph = (uint32_t)(i / S) & 1u;
-          mb_wait(&full_bar[s], ph);
+          mbarrier_wait<S_SPIN_LOG2>(&full_bar[s], ph);
           uint8_t* st = smem + (size_t)s * stage_bytes;
           for (uint32_t q0 = tid; q0 < n16; q0 += 4 * S_WORKERS) {   // 4 granules in flight per thread
             uint4 v[4];
@@ -332,12 +246,12 @@ tc3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CU
               }
             }
           }
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic writes -> visible to the MMA (async proxy)
-          mb_arrive(&conv_bar[s]);
+          fence_proxy_async_shared();   // generic writes -> visible to the MMA (async proxy)
+          mbarrier_arrive(&conv_bar[s]);
         }
       }
-      mb_wait(tmem_full_bar, 0);
-      tcf_after();
+      mbarrier_wait<S_SPIN_LOG2>(tmem_full_bar, 0);
+      tcgen05_fence_after();
       const int quarter = warp & 3;                   // TMEM lane quarter this warp may read
       const int half = (warp - 2) >> 2;               // the two warps of a quarter split the columns
       const int rloc = quarter * 32 + lane;
@@ -349,15 +263,15 @@ tc3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CU
       const int c_begin = half ? c_split : 0, c_end = half ? NT : c_split;
       // 16 accumulator columns of this thread's row: main (+ cross-term accumulator)
       auto load16 = [&](int c, float (&v)[16]) {
-        tmem_ld16(taddr + c, v);
+        tcgen05_ld_32x32b_x16(taddr + c, v);
         if (split) {
           float w[16];
-          tmem_ld16(taddr + lo_col + c, w);
-          tmem_ld_wait();
+          tcgen05_ld_32x32b_x16(taddr + lo_col + c, w);
+          tcgen05_wait_ld();
 #pragma unroll
           for (int j = 0; j < 16; ++j) v[j] += w[j];
         } else {
-          tmem_ld_wait();
+          tcgen05_wait_ld();
         }
       };
 
@@ -394,7 +308,7 @@ tc3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CU
             if (++t == W) { t = 0; ++bl; }
           }
         }
-        asm volatile("bar.sync 1, 256;" ::: "memory");
+        bar_sync<1, 256>();
         const int nv = min(S_BM, g.M - m0);                 // valid rows of this tile
         const int nbl = NT / W;                             // batch elements per tile (NT is a multiple of W)
         const int b0 = n0 / W;
@@ -421,8 +335,8 @@ tc3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CU
                 const int mp = m0 + rl, node = mp / 3, kp = mp - node * 3;
                 const float4 f = *reinterpret_cast<const float4*>(src + rl * W + 4 * u);
                 unsigned short h0, h1, h2, h3, l0, l1, l2, l3;
-                to_h16(f.x, g.bf16, h0, l0); to_h16(f.y, g.bf16, h1, l1);
-                to_h16(f.z, g.bf16, h2, l2); to_h16(f.w, g.bf16, h3, l3);
+                split_f16_hi_lo(f.x, g.bf16, h0, l0); split_f16_hi_lo(f.y, g.bf16, h1, l1);
+                split_f16_hi_lo(f.z, g.bf16, h2, l2); split_f16_hi_lo(f.w, g.bf16, h3, l3);
                 const size_t o = ((size_t)b * Nn + node) * g.ldh + kp * W + 4 * u;
                 *reinterpret_cast<uint2*>(g.g_hi + o) =
                     make_uint2((uint32_t)h0 | ((uint32_t)h1 << 16), (uint32_t)h2 | ((uint32_t)h3 << 16));
@@ -435,7 +349,7 @@ tc3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CU
                 const int rl = it / W, t = it - rl * W;
                 const int mp = m0 + rl, node = mp / 3, kp = mp - node * 3;
                 unsigned short hh, ll;
-                to_h16(src[it], g.bf16, hh, ll);
+                split_f16_hi_lo(src[it], g.bf16, hh, ll);
                 const size_t o = ((size_t)b * Nn + node) * g.ldh + kp * W + t;
                 g.g_hi[o] = hh;
                 if (!g.bf16) g.g_lo[o] = ll;
@@ -464,7 +378,7 @@ tc3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CU
         const bool has_bc = g.bc_bnw != nullptr;
         if (valid && has_bc && half == 0)
           for (int t = 0; t < W; ++t) s_x[t * 128 + rloc] = g.x_bnw[(long long)row * W + t];
-        asm volatile("bar.sync 1, 256;" ::: "memory");     // a row's columns were produced by two warps
+        bar_sync<1, 256>();     // a row's columns were produced by two warps
         if (valid) {
           const int b = row / g.Nn, node = row - b * g.Nn;
           const int o_split = (W + 1) / 2;
@@ -489,42 +403,12 @@ tc3_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CU
       }
     }
   }
-  tcf_before();
+  tcgen05_fence_before();
   __syncthreads();
   if (warp == 1) {
-    tcf_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(g.tmem_cols) : "memory");
+    tcgen05_fence_after();
+    tcgen05_dealloc(tmem_base, g.tmem_cols);
   }
-}
-
-typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                             const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                             CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeFn encode_fn() {
-  static EncodeFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) == cudaSuccess &&
-        q == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeFn>(p);
-    else
-      (void)cudaGetLastError();
-  }
-  return fn;
-}
-// 2-D fp32 tensor: `rows` x `cols` logical extent (anything outside reads as zero), row pitch ld floats (ld % 4 == 0);
-// box = box_rows x 32 columns, 128B swizzle
-bool map_f32(EncodeFn enc, CUtensorMap* map, const float* base, int rows, int cols, int ld, int box_rows) {
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * sizeof(float)};
-  cuuint32_t box[2] = {(cuuint32_t)S_BK, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, estr,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
 uint32_t pow2_cols(int n) {
@@ -607,10 +491,12 @@ int tc3_gemm(int M, int N, int K, float alpha, const float* A, int lda, const fl
              float* C1, int msplit, int ldc, int n_store, int atomic, int splits, int split_ops, cudaStream_t st) {
   if (N % 16 != 0 || N < 16 || N > 256 || K < 1 || (lda & 3) != 0 || (ldb & 3) != 0) return -1;
   if (!aligned16(A) || !aligned16(B)) return -1;
-  EncodeFn enc = encode_fn();
-  if (enc == nullptr) return -1;
   CUtensorMap ma, mb;
-  if (!map_f32(enc, &ma, A, M, K, lda, S_BM) || !map_f32(enc, &mb, B, n_rows_b, K, ldb, N)) return -1;
+  if (!make_tensor_map_2d(&ma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, A, M, K, lda * 4ull, S_BM, S_BK,
+                          CU_TENSOR_MAP_SWIZZLE_128B) ||
+      !make_tensor_map_2d(&mb, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, B, n_rows_b, K, ldb * 4ull, N, S_BK,
+                          CU_TENSOR_MAP_SWIZZLE_128B))
+    return -1;
   size_t smem = 0;
   const int ns = plan_smem(N, split_ops, 0, 0, 4, &smem);
   if (ns == 0) return -1;
@@ -632,14 +518,16 @@ int gft_tc(const float* mul_Lp, int ldl, const float* xp, int ldx, float* G, uns
   if (off || mul_Lp == nullptr || xp == nullptr) return -1;
   if ((ldl & 3) != 0 || (ldx & 3) != 0 || !aligned16(mul_Lp) || !aligned16(xp)) return -1;
   if (g_img != nullptr && ((ldh & 1) != 0 || ldh < 3 * W)) return -1;
-  EncodeFn enc = encode_fn();
-  if (enc == nullptr) return -1;
   // column tile = whole batch elements (the epilogue writes G[b][tile rows][0..W) as one dense block per b)
   const int NT = lcm_i(W, 16);
   if (NT > 128) return -1;
   const int M = 3 * N, BW = B * W;
   CUtensorMap ma, mb;
-  if (!map_f32(enc, &ma, mul_Lp, M, N, ldl, S_BM) || !map_f32(enc, &mb, xp, BW, N, ldx, NT)) return -1;
+  if (!make_tensor_map_2d(&ma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, mul_Lp, M, N, ldl * 4ull, S_BM, S_BK,
+                          CU_TENSOR_MAP_SWIZZLE_128B) ||
+      !make_tensor_map_2d(&mb, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, xp, BW, N, ldx * 4ull, NT, S_BK,
+                          CU_TENSOR_MAP_SWIZZLE_128B))
+    return -1;
   size_t smem = 0;
   const int ns = plan_smem(NT, split_ops, 0, (size_t)S_BM * NT * sizeof(float), 4, &smem);   // ring doubles as the staging tile
   if (ns == 0) return -1;
@@ -660,10 +548,12 @@ int out_head_tc(const float* act3, int K, const float* woutT, int PWp, const Hea
   const int T = h.T, W = h.W, R = h.R;
   if (PWp % 16 != 0 || PWp < 16 || PWp > 256 || (K & 3) != 0 || !aligned16(act3) || !aligned16(woutT)) return -1;
   if (PWp < T + (h.backcast_bnw != nullptr ? W : 0)) return -1;
-  EncodeFn enc = encode_fn();
-  if (enc == nullptr) return -1;
   CUtensorMap ma, mb;
-  if (!map_f32(enc, &ma, act3, R, K, K, S_BM) || !map_f32(enc, &mb, woutT, PWp, K, K, PWp)) return -1;
+  if (!make_tensor_map_2d(&ma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, act3, R, K, K * 4ull, S_BM, S_BK,
+                          CU_TENSOR_MAP_SWIZZLE_128B) ||
+      !make_tensor_map_2d(&mb, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, woutT, PWp, K, K * 4ull, PWp, S_BK,
+                          CU_TENSOR_MAP_SWIZZLE_128B))
+    return -1;
   const size_t extra = sizeof(float) * ((size_t)W * T + (size_t)W * W + T + 3 * (size_t)W + (size_t)(T + 2 * W) * 128) + 64;
   size_t smem = 0;
   const int ns = plan_smem(PWp, split_ops, extra, 0, 4, &smem);
